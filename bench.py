@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- env-steps/s of the rollout hot path (crowd step + DS-RNN forward) on N B200s.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c3|c2|c1] [--precision fp32|bf16x3|bf16]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c3|c2|c1] [--precision fp32|bf16x3|bf16] [--dump-outputs DIR]
     python bench.py --impl reference ...      # the CPU arm: the oracle port on the box's host cores
 
 One "step" = Policy.act (DS-RNN forward, deterministic) + CrowdSimDict.step for every env of the batch
@@ -18,6 +18,7 @@ import json
 import os
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -111,6 +112,29 @@ def load_weights(name):
     path = os.path.join(ROOT, "tests", "golden", "weights_%s.npz" % name)
     w = np.load(path)
     return {k: w[k] for k in w.files}
+
+
+DUMP_BYTES = 64 * 10 ** 6      # --dump-outputs writes at most this much in all
+
+
+def dump_outputs(path, arrays, n_envs=None):
+    """--dump-outputs: write each array (torch tensor or numpy) as <path>/<name>.npy, float64 as float64 and everything else as
+    float32.  If they would exceed DUMP_BYTES together, every array whose first axis is the env axis (length n_envs) keeps
+    the same fixed, seeded sample of envs, so that two runs with the same arguments write the same rows."""
+    out = {}
+    for name, a in arrays.items():
+        a = a.detach().cpu().numpy() if hasattr(a, "detach") else np.asarray(a)
+        out[name] = a if a.dtype == np.float64 else a.astype(np.float32)
+    per_env = lambda a: n_envs is not None and a.ndim > 0 and a.shape[0] == n_envs
+    env_bytes = sum(a.nbytes for a in out.values() if per_env(a))
+    budget = DUMP_BYTES - 128 * len(out) - sum(a.nbytes for a in out.values() if not per_env(a))     # 128 B: .npy header
+    if env_bytes > budget:
+        keep = max(1, int(budget // (env_bytes // n_envs)))
+        rows = np.sort(np.random.default_rng(0).choice(n_envs, keep, replace=False))
+        out = {k: a[rows] if per_env(a) else a for k, a in out.items()}
+    os.makedirs(path, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(path, name + ".npy"), a)
 
 
 class ClockSampler(threading.Thread):
@@ -252,11 +276,15 @@ def run_ours(args, wl):
         torch.cuda.synchronize()
 
     # ---------------- device-resident rollout (value)
+    last = {}       # what the last step of the last rollout() call returned (--dump-outputs of the eager loop)
+
     def rollout(steps, obs, hx, masks):
         for _ in range(steps):
-            _, action, _, hx = policy.act(obs, hx, masks, deterministic=True)
-            obs, _, done, _ = venv.step_device(action)
+            value, action, _, hx = policy.act(obs, hx, masks, deterministic=True)
+            obs, reward, done, _ = venv.step_device(action)
             masks = (1.0 - done.to(torch.float32)).unsqueeze(1)
+        if steps:
+            last.update(obs, reward=reward, done=done, value=value, action=action, **hx)
         return obs, hx, masks
 
     obs = venv.reset()
@@ -278,6 +306,8 @@ def run_ours(args, wl):
         obs, hx, masks = rollout(args.steps, obs, hx, masks)
         ev1.record()
         barrier()
+        if args.dump_outputs and rank == 0:
+            dump_outputs(args.dump_outputs, last, N)
         launches = eng.launches + policy.gpu_launches - launches0
     else:
         # the timed loop replays the rollout step (crowd step incl. swap-in of spare episodes -> forward on the new observation,
@@ -295,6 +325,12 @@ def run_ours(args, wl):
             buf = roll.step()
         ev1.record()
         barrier()
+        if args.dump_outputs and rank == 0:
+            # the last replay stepped the envs into `buf`, then ran the forward on that observation: it wrote action and value to
+            # sets[parity] and the hidden state it produced to sets[parity ^ 1] (GraphedRollout._one_step)
+            fw, h = roll.sets[roll.parity], roll.sets[roll.parity ^ 1]
+            dump_outputs(args.dump_outputs, dict(buf.obs(), reward=buf.reward, done=buf.done, value=fw["value"], action=fw["mean"],
+                                                 human_node_rnn=h["h_node"], human_human_edge_rnn=h["h_edge"]), N)
         launches = args.steps * roll.launches_per_step
         # per-kernel durations for the roofline: CUDA events recorded by the library around the dominant kernels on the
         # launching stream, over a short EAGER continuation of the same step schedule (events cannot be read back from a
@@ -509,6 +545,9 @@ def run_train(args, wl):
         losses = cycle()
     e1.record()
     barrier()
+    if args.dump_outputs and rank == 0:
+        # the last update cycle returned the averaged losses (value, action, entropy) and left the updated weights in the policy
+        dump_outputs(args.dump_outputs, dict(losses=losses, **{"param." + k: v for k, v in policy.state_dict().items()}))
     ms = e0.elapsed_time(e1)
     launches = venv.engine.launches + policy.gpu_launches + native.COUNTERS["gemm_launches"] + native.COUNTERS["kernel_launches"] - launches0
     clocks = sampler.stop() if rank == 0 else None
@@ -532,12 +571,14 @@ def run_train(args, wl):
     barrier()
     t0 = torch.cuda.Event(enable_timing=True)
     t1 = torch.cuda.Event(enable_timing=True)
-    train_api(cfg, dev, num_updates=1, output_dir=None, actor_critic=policy, log=None, max_envs_per_pass=per_pass, native_update=True)
-    barrier()
-    t0.record()
-    train_api(cfg, dev, num_updates=e2e_updates, output_dir=None, actor_critic=policy, log=None, max_envs_per_pass=per_pass, native_update=True)
-    t1.record()
-    barrier()
+    # train() writes its run artefacts (configs, log, progress.csv, checkpoint) like a user's run does, but not into the tree
+    with tempfile.TemporaryDirectory() as run_dir:
+        train_api(cfg, dev, num_updates=1, output_dir=run_dir, actor_critic=policy, log=None, max_envs_per_pass=per_pass, native_update=True)
+        barrier()
+        t0.record()
+        train_api(cfg, dev, num_updates=e2e_updates, output_dir=run_dir, actor_critic=policy, log=None, max_envs_per_pass=per_pass, native_update=True)
+        t1.record()
+        barrier()
     e2e_ms = t0.elapsed_time(t1)
     if world > 1:
         t = torch.tensor([ms, e2e_ms], device=dev)
@@ -619,8 +660,16 @@ def main():
     ap.add_argument("--no-graph", action="store_true", help="time the eager loop instead of the CUDA-graph replay")
     ap.add_argument("--envs-total", type=int, default=0, help="c5: total envs over all GPUs (default 65536)")
     ap.add_argument("--envs-per-pass", type=int, default=4096, help="c5: env trajectories per forward/backward pass of the update")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (float32 / float64, at most "
+                         "64 MB: a fixed sample of envs when larger; rank 0's envs): c1-c3 the observation, reward, done, value, "
+                         "action and hidden state of the step, c5 the losses and the updated weights")
     args = ap.parse_args()
     wl = WORKLOADS[args.workload]
+    if args.steps is not None and args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of this project's GPU path; --impl reference has none")
     if args.steps is None:
         args.steps = 3 if wl.get("train") else 200
     if args.warmup is None:

@@ -34,6 +34,25 @@ def test_own_arm_line_has_every_contract_key():
     assert set(d["clocks"]) >= {"sm_mhz", "sm_max_mhz", "reasons"}
 
 
+def test_dump_outputs_of_the_last_timed_step(tmp_path):
+    """--dump-outputs: the same arguments give the same arrays; one more timed step gives another state."""
+    import numpy as np
+
+    dumps = {}
+    for name, steps in (("a", "6"), ("b", "6"), ("c", "7")):
+        d = _run("--dump-outputs", str(tmp_path / name), "--steps", steps, "--no-cpu-baseline")
+        assert d["steps"] == int(steps)
+        files = sorted(os.listdir(tmp_path / name))
+        dumps[name] = {f[:-4]: np.load(tmp_path / name / f) for f in files}
+        assert sum(os.path.getsize(tmp_path / name / f) for f in files) <= 64 * 10 ** 6
+    a, b, c = dumps["a"], dumps["b"], dumps["c"]
+    assert sorted(a) == ["action", "done", "human_human_edge_rnn", "human_node_rnn", "reward", "robot_node", "spatial_edges",
+                         "temporal_edges", "value"]
+    assert all(v.dtype == np.float32 and v.shape[0] == 16 for v in a.values())
+    assert all(np.array_equal(a[k], b[k]) for k in a)
+    assert not np.array_equal(a["robot_node"], c["robot_node"])
+
+
 def test_reference_arm_line():
     d = _run("--impl", "reference")
     assert d["impl"] == "reference" and d["value"] > 0 and d["gpu_launches"] == 0

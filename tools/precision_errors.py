@@ -1,5 +1,6 @@
 import os, sys, numpy as np, torch
-sys.path.insert(0, '/root/repo'); sys.path.insert(0, '/root/repo/tests')
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, "tests"))
 from helpers import DSRNN_CASES, GOLDEN
 from test_gpu_dsrnn import _policy, _rel_err
 for prec in ("bf16x3", "fp16", "bf16"):
