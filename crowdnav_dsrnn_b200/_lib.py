@@ -50,6 +50,10 @@ SYMBOLS = {
     "cn_gru_gates_backward_pairs": (C.c_int, [_P, _P, C.c_int, _P, _P, _P, _P, _P, _P, C.c_int, C.c_int, _P]),
     "cn_gemm_bf16x3": (C.c_int, [C.POINTER(abi.CnGemm), C.c_int, _P]),
     "cn_encoder_grad": (C.c_int, [_P, _P, C.c_int, _P, _P, _P, C.c_longlong, _P]),
+    "cn_encoder_grad_ordered_workspace_bytes": (C.c_size_t, [C.c_longlong]),
+    "cn_encoder_grad_ordered": (C.c_int, [_P, _P, C.c_int, _P, _P, _P, C.c_longlong, _P, C.c_size_t, _P]),
+    "cn_gemm_bf16x3_ordered_workspace_bytes": (C.c_int, [C.POINTER(abi.CnGemm), C.c_int, C.POINTER(C.c_size_t), C.POINTER(C.c_int)]),
+    "cn_gemm_bf16x3_ordered": (C.c_int, [C.POINTER(abi.CnGemm), C.c_int, _P, C.c_size_t, _P]),
     "cn_gemm_enable_timing": (C.c_int, [C.c_int]),
     "cn_gemm_time_ms": (C.c_int, [C.POINTER(C.c_float), C.POINTER(C.c_int), C.POINTER(C.c_double)]),
     "cn_attention_train_forward": (C.c_int, [_P, _P, _P, _P, _P, C.c_float, C.c_int, C.c_int, _P]),

@@ -454,7 +454,9 @@ extern "C" int cn_split_bf16(const float *a, void *hi, void *lo, size_t n, void 
 extern "C" int cn_launch_gru_gates_backward_pairs(const float *grad_h, float *d, int d_live, const float *m_next, const float *ws,
                                                   const float *h_prev, const float *m_cur, void *g_hi, void *g_lo, int R, int hid,
                                                   cudaStream_t stream);
-const char *gemm_bf16x3_launch(const CnGemm *problems, int n_problems, cudaStream_t stream, int *items_out);
+const char *gemm_bf16x3_launch(const CnGemm *problems, int n_problems, cudaStream_t stream, int *items_out, bool ordered,
+                               void *workspace, size_t workspace_bytes);
+const char *gemm_bf16x3_ordered_workspace(const CnGemm *problems, int n_problems, size_t *bytes, int *slices);
 
 extern "C" int cn_gru_gates_backward_pairs(const float *grad_h, float *d, int d_live, const float *m_next, const float *ws,
                                            const float *h_prev, const float *m_cur, void *g_hi, void *g_lo, int rows, int hid, void *stream)
@@ -469,8 +471,24 @@ extern "C" int cn_gru_gates_backward_pairs(const float *grad_h, float *d, int d_
 extern "C" int cn_gemm_bf16x3(const CnGemm *problems, int n_problems, void *stream)
 {
     if (!problems) return fail(CN_ERR_ARG, "cn_gemm_bf16x3: problems is NULL");
-    const char *msg = gemm_bf16x3_launch(problems, n_problems, (cudaStream_t)stream, nullptr);
+    const char *msg = gemm_bf16x3_launch(problems, n_problems, (cudaStream_t)stream, nullptr, false, nullptr, 0);
     if (msg) return fail(CN_ERR_ARG, "cn_gemm_bf16x3: %s", msg);
+    return CN_OK;
+}
+
+extern "C" int cn_gemm_bf16x3_ordered_workspace_bytes(const CnGemm *problems, int n_problems, size_t *bytes, int *slices)
+{
+    if (!problems || !bytes) return fail(CN_ERR_ARG, "cn_gemm_bf16x3_ordered_workspace_bytes: NULL pointer");
+    const char *msg = gemm_bf16x3_ordered_workspace(problems, n_problems, bytes, slices);
+    if (msg) return fail(CN_ERR_ARG, "cn_gemm_bf16x3_ordered_workspace_bytes: %s", msg);
+    return CN_OK;
+}
+
+extern "C" int cn_gemm_bf16x3_ordered(const CnGemm *problems, int n_problems, void *workspace, size_t workspace_bytes, void *stream)
+{
+    if (!problems) return fail(CN_ERR_ARG, "cn_gemm_bf16x3_ordered: problems is NULL");
+    const char *msg = gemm_bf16x3_launch(problems, n_problems, (cudaStream_t)stream, nullptr, true, workspace, workspace_bytes);
+    if (msg) return fail(CN_ERR_ARG, "cn_gemm_bf16x3_ordered: %s", msg);
     return CN_OK;
 }
 
@@ -529,5 +547,22 @@ extern "C" int cn_encoder_grad(const float *de, const void *e_hi, int ld_e, cons
     const int rc = cn_launch_encoder_grad(de, e_hi, ld_e, x, dw, db, rows, (cudaStream_t)stream);
     if (rc == -1) return fail(CN_ERR_ARG, "cn_encoder_grad: rows %lld / ld_e %d (>= 64) / alignment", rows, ld_e);
     if (rc != 0) return fail(CN_ERR_CUDA, "encoder_grad_kernel: %s", cudaGetErrorString((cudaError_t)rc));
+    return CN_OK;
+}
+
+extern "C" size_t cn_launch_encoder_grad_ordered_bytes(long long rows);
+extern "C" int cn_launch_encoder_grad_ordered(const float *de, const void *e_hi, int ld_e, const float *x, float *dw, float *db, long long rows,
+                                              void *workspace, size_t workspace_bytes, cudaStream_t stream);
+extern "C" size_t cn_encoder_grad_ordered_workspace_bytes(long long rows) { return cn_launch_encoder_grad_ordered_bytes(rows); }
+extern "C" int cn_encoder_grad_ordered(const float *de, const void *e_hi, int ld_e, const float *x, float *dw, float *db, long long rows,
+                                       void *workspace, size_t workspace_bytes, void *stream)
+{
+    if (!de || !e_hi || !x || !dw || !db) return fail(CN_ERR_ARG, "cn_encoder_grad_ordered: NULL pointer");
+    const int rc = cn_launch_encoder_grad_ordered(de, e_hi, ld_e, x, dw, db, rows, workspace, workspace_bytes, (cudaStream_t)stream);
+    if (rc == -1) return fail(CN_ERR_ARG, "cn_encoder_grad_ordered: rows %lld / ld_e %d (>= 64) / alignment", rows, ld_e);
+    if (rc == -2)
+        return fail(CN_ERR_ARG, "cn_encoder_grad_ordered: workspace NULL, not 16-byte aligned or smaller than %zu bytes (%zu given)",
+                    cn_launch_encoder_grad_ordered_bytes(rows), workspace_bytes);
+    if (rc != 0) return fail(CN_ERR_CUDA, "encoder_grad_kernel (ordered): %s", cudaGetErrorString((cudaError_t)rc));
     return CN_OK;
 }

@@ -251,10 +251,12 @@ attention_train_backward_kernel(const float *__restrict__ o, const float *__rest
 // e = ReLU(W_enc x + b) with x [rows, 2] (HumanHumanEdgeRNN.encoder_linear, srnn_model.py:201-215).  Given de = dL/de
 // [rows, 64] (fp32) and the sign of e (its bf16 hi image, row stride ld_e):  dW_enc[k, j] = sum_rows [e_k > 0] de_k x_j,
 // db_enc[k] = sum_rows [e_k > 0] de_k.  One pass over de: HBM-bound.  Block = 4 rows x 64 columns per iteration; block sums are
-// combined in shared memory and added to the outputs with 64 x 3 atomics per block.
+// combined in shared memory and added to the outputs with 64 x 3 atomics per block.  The ordered instantiation writes the
+// 64 x 3 block sums to part[block] instead, and encoder_grad_reduce_kernel adds them to dw / db in block order.
+template <bool kOrdered>
 __global__ void __launch_bounds__(256)
 encoder_grad_kernel(const float *__restrict__ de, const __nv_bfloat16 *__restrict__ e_hi, int ld_e, const float *__restrict__ x,
-                    float *__restrict__ dw, float *__restrict__ db, long long rows)
+                    float *__restrict__ dw, float *__restrict__ db, long long rows, float *__restrict__ part_out)
 {
     __shared__ float part[4][64][3];
     const int col = threadIdx.x & 63, rsub = threadIdx.x >> 6;
@@ -270,8 +272,28 @@ encoder_grad_kernel(const float *__restrict__ de, const __nv_bfloat16 *__restric
     if (threadIdx.x < 192) {
         const int c = threadIdx.x / 3, k = threadIdx.x - 3 * c;
         const float t = part[0][c][k] + part[1][c][k] + part[2][c][k] + part[3][c][k];
-        if (k < 2) atomicAdd(dw + c * 2 + k, t); else atomicAdd(db + c, t);
+        if (kOrdered) part_out[(size_t)blockIdx.x * 192 + threadIdx.x] = t;
+        else if (k < 2) atomicAdd(dw + c * 2 + k, t); else atomicAdd(db + c, t);
     }
+}
+
+// dw[c, k] (k < 2) / db[c] (k = 2) += part[0][c][k] + part[1][c][k] + ... in block order; one thread per output
+__global__ void __launch_bounds__(192)
+encoder_grad_reduce_kernel(const float *__restrict__ part, int blocks, float *__restrict__ dw, float *__restrict__ db)
+{
+    const int t = threadIdx.x, c = t / 3, k = t - 3 * c;
+    float *out = k < 2 ? dw + c * 2 + k : db + c;
+    float acc = *out;
+#pragma unroll 16
+    for (int b = 0; b < blocks; ++b) acc += part[(size_t)b * 192 + t];
+    *out = acc;
+}
+
+// grid of encoder_grad_kernel: a function of `rows` only
+inline long long encoder_grad_blocks(long long rows)
+{
+    const long long blocks = (rows + 3) / 4;
+    return blocks < 148 * 8 ? blocks : 148 * 8;
 }
 
 inline bool aligned16(const void *p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
@@ -353,8 +375,28 @@ extern "C" int cn_launch_encoder_grad(const float *de, const void *e_hi, int ld_
                                       cudaStream_t stream)
 {
     if (rows < 1 || ld_e < 64 || !aligned16(de) || !aligned8(x)) return -1;
-    long long blocks = (rows + 3) / 4;
-    if (blocks > 148 * 8) blocks = 148 * 8;
-    encoder_grad_kernel<<<(unsigned)blocks, 256, 0, stream>>>(de, static_cast<const __nv_bfloat16 *>(e_hi), ld_e, x, dw, db, rows);
+    const long long blocks = encoder_grad_blocks(rows);
+    encoder_grad_kernel<false><<<(unsigned)blocks, 256, 0, stream>>>(de, static_cast<const __nv_bfloat16 *>(e_hi), ld_e, x, dw, db, rows,
+                                                                     nullptr);
+    return (int)cudaGetLastError();
+}
+
+extern "C" size_t cn_launch_encoder_grad_ordered_bytes(long long rows)
+{
+    return rows < 1 ? 0 : (size_t)encoder_grad_blocks(rows) * 192 * sizeof(float);
+}
+
+// -1 bad arguments, -2 workspace NULL / misaligned / too small
+extern "C" int cn_launch_encoder_grad_ordered(const float *de, const void *e_hi, int ld_e, const float *x, float *dw, float *db, long long rows,
+                                              void *workspace, size_t workspace_bytes, cudaStream_t stream)
+{
+    if (rows < 1 || ld_e < 64 || !aligned16(de) || !aligned8(x)) return -1;
+    if (!workspace || !aligned16(workspace) || workspace_bytes < cn_launch_encoder_grad_ordered_bytes(rows)) return -2;
+    const long long blocks = encoder_grad_blocks(rows);
+    float *part = static_cast<float *>(workspace);
+    encoder_grad_kernel<true><<<(unsigned)blocks, 256, 0, stream>>>(de, static_cast<const __nv_bfloat16 *>(e_hi), ld_e, x, dw, db, rows, part);
+    const cudaError_t err = cudaGetLastError();
+    if (err != cudaSuccess) return (int)err;
+    encoder_grad_reduce_kernel<<<1, 192, 0, stream>>>(part, (int)blocks, dw, db);
     return (int)cudaGetLastError();
 }

@@ -3,7 +3,7 @@
 // srnn_model.py:53-104 and its autograd transpose): forward linears, the recurrent products of the masked GRU sequences
 // and their backward, and the weight-gradient reductions over the T*R row dimension.
 //
-//     C[M,N] (fp32)   =  | +=  | atomically +=     (A_hi + A_lo)(B_hi + B_lo)   (+ bias[n], ReLU / tanh)
+//     C[M,N] (fp32)   =  | +=  | split-K: += partial products     (A_hi + A_lo)(B_hi + B_lo)   (+ bias[n], ReLU / tanh)
 //
 // Split-bf16 3-pass arithmetic (A_hi B_hi + A_lo B_hi + A_hi B_lo, fp32 accumulation in TMEM; operand error ~2^-16: the
 // precision of the rollout kernels, CN_PREC_BF16X3).  Operands are bf16 (hi, lo) pairs in global memory, written by the
@@ -21,6 +21,10 @@
 //   warps 2-9   epilogue: tcgen05.ld -> (bias, activation) -> 256-bit stores of each lane's row segment, read-modify-write
 //               (accumulate) or red.global.add (split-K partial sums), overlapped with the MMAs of the next item through
 //               the second TMEM buffer.
+// Ordered split-K (cn_gemm_bf16x3_ordered, the `kOrdered` instantiation): a k-slice stores its partial tile into its own
+// slice of a caller-provided workspace instead (every element written once, by one CTA: no atomics, no inter-CTA waits),
+// and splitk_reduce_kernel then forms C = C_in + P_0 + ... + P_{S-1} in slice order.  The slice count is a function of the
+// problem's own (m, n, k, split_k) only (ordered_slices), so a product gives the same bits alone or grouped, on any device.
 // CTAs are launched as clusters of c = 1, 2 or 4 that walk c consecutive 128-row tiles of the same (k-slice, n-tile) in lock
 // step: the B tile (weights: the same for every row tile, and the larger operand of the recurrent products) is fetched from
 // L2 once per cluster -- every CTA loads 1/c of it and TMA-multicasts it into all c shared memories
@@ -60,7 +64,7 @@ struct alignas(64) GemmProblem {
     int split_k, kb_per_split; // k-blocks (64 deep) per k-slice
     int a_mn, b_mn;            // operand majors (1 = MN-major)
     int a_lo_on, b_lo_on;      // passes A_lo*B_hi / A_hi*B_lo enabled
-    int act, mode;             // mode 0 store, 1 read-modify-write add, 2 atomic add
+    int act, mode;             // mode 0 store, 1 read-modify-write add, 2 atomic add, 3 store into workspace slice ks (ordered)
     int m_groups;              // groups of c consecutive m-tiles (one per cluster and item)
     int b_slice_bytes;         // bytes of one CTA's slice of the B tile (K-major: bn/c rows; MN-major: 64/c k-rows of every atom)
     int item0, items;          // this problem's range of global work items (one item = one cluster-wide group of m-tiles)
@@ -128,6 +132,7 @@ __device__ __forceinline__ Item decode_item(const GemmArgs &a, int item, int ran
     return it;
 }
 
+template <bool kOrdered>
 __global__ void __launch_bounds__(kThreads, 1) gemm_bf16x3_kernel(const __grid_constant__ GemmArgs a)
 {
     extern __shared__ unsigned char smem_dyn[];
@@ -290,7 +295,8 @@ __global__ void __launch_bounds__(kThreads, 1) gemm_bf16x3_kernel(const __grid_c
             const int mode = g.mode, act = g.act;
             if (it.mt * kTileM + q * 32 < g.m) {              // else padding rows (ragged last tile / last group): nothing to store
                 const bool row_ok = m < g.m;
-                float *crow = g.c + (size_t)(row_ok ? m : 0) * g.ldc + col0;
+                // (mode 3: c is slice 0 of this problem's workspace, [m, ldc] per slice)
+                float *crow = g.c + (kOrdered && mode == 3 ? (size_t)it.ks * g.m * g.ldc : 0) + (size_t)(row_ok ? m : 0) * g.ldc + col0;
                 const bool fast = ((g.ldc & 7) == 0) && ((reinterpret_cast<uintptr_t>(g.c) & 31) == 0) && ((col0 & 7) == 0);
                 for (int cb = half; cb * 32 < ncols; cb += 2) {
                     const int c0 = cb * 32;
@@ -303,7 +309,7 @@ __global__ void __launch_bounds__(kThreads, 1) gemm_bf16x3_kernel(const __grid_c
                         for (int j = 16; j < 32; ++j) acc[j] = 0.f;
                     }
                     tmem_ld_wait();
-                    if (mode == 2) {                          // split-K partial sums
+                    if (!kOrdered && mode == 2) {             // split-K partial sums
                         if (row_ok) {
 #pragma unroll
                             for (int j = 0; j < 32; ++j)
@@ -357,6 +363,58 @@ __global__ void __launch_bounds__(kThreads, 1) gemm_bf16x3_kernel(const __grid_c
     }
 }
 
+// Ordered split-K reduction: C = C_in + P_0 + P_1 + ... + P_{S-1}, summed left to right in fp32, for every split problem of
+// one ordered launch.  P_s is [m, n_pad] (n_pad = n rounded up to 8) at p + s * m * n_pad.  One thread per 4 columns of a row:
+// float4 loads of the partials (read once: evict-first), float4 read-modify-write of C where its layout allows it.
+struct ReduceProblem {
+    float *c;
+    const float *p;
+    long long ldc;
+    long long unit0;           // first unit (4 columns of a row) of this problem in the launch
+    int m, n, n_pad, slices, vec;
+};
+struct ReduceArgs {
+    ReduceProblem p[kMaxProblems];
+    int n_problems;
+    long long total_units;
+};
+
+__global__ void __launch_bounds__(256) splitk_reduce_kernel(const __grid_constant__ ReduceArgs a)
+{
+    for (long long u = (long long)blockIdx.x * blockDim.x + threadIdx.x; u < a.total_units; u += (long long)gridDim.x * blockDim.x) {
+        int i = 0;
+        while (i + 1 < a.n_problems && u >= a.p[i + 1].unit0) ++i;
+        const ReduceProblem &g = a.p[i];
+        const long long r = u - g.unit0;
+        const int q4 = g.n_pad >> 2;
+        const int row = (int)(r / q4), col = (int)(r - (long long)row * q4) << 2;
+        const int nv = g.n - col < 4 ? g.n - col : 4;
+        if (nv <= 0) continue;
+        const size_t slice = (size_t)g.m * g.n_pad;
+        const float *src = g.p + (size_t)row * g.n_pad + col;
+        float *dst = g.c + (size_t)row * g.ldc + col;
+        float acc[4] = {0.f, 0.f, 0.f, 0.f};
+        const bool v4 = g.vec && nv == 4;
+        if (v4) {
+            const float4 t = *reinterpret_cast<const float4 *>(dst);
+            acc[0] = t.x; acc[1] = t.y; acc[2] = t.z; acc[3] = t.w;
+        } else {
+#pragma unroll
+            for (int j = 0; j < 4; ++j) if (j < nv) acc[j] = dst[j];
+        }
+        for (int s = 0; s < g.slices; ++s) {
+            const float4 t = __ldcs(reinterpret_cast<const float4 *>(src + s * slice));
+            acc[0] += t.x; acc[1] += t.y; acc[2] += t.z; acc[3] += t.w;
+        }
+        if (v4) {
+            *reinterpret_cast<float4 *>(dst) = make_float4(acc[0], acc[1], acc[2], acc[3]);
+        } else {
+#pragma unroll
+            for (int j = 0; j < 4; ++j) if (j < nv) dst[j] = acc[j];
+        }
+    }
+}
+
 typedef CUresult (*EncodeTiled)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *, const cuuint64_t *,
                                 const cuuint32_t *, const cuuint32_t *, CUtensorMapInterleave, CUtensorMapSwizzle,
                                 CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
@@ -406,6 +464,54 @@ static int pick_cluster(const GemmArgs &args, int n_problems, int forced)
     return 1;
 }
 
+// n-tile of a problem: n rounded up to 16 up to 256; wider problems get even n-tiles (e.g. 320 -> 2 x 160) instead of a
+// full tile and a sliver
+static int tile_n(int n)
+{
+    if (n <= 256) return (n + 15) & ~15;
+    const int tiles = (n + 255) / 256;
+    return (((n + tiles - 1) / tiles) + 15) & ~15;
+}
+
+// Slice count of a problem in ordered mode: a pure function of its own (m, n, k, split_k).  split_k = 0 evaluates the auto
+// rule of gemm_bf16x3_launch below for the problem alone (share 1) with a fixed budget of 74 clusters of 2 (148 SMs, a
+// B200), so that neither the device, the cluster choice nor the other problems of a launch change the summation order.
+static constexpr int kOrderedClusters = 74, kOrderedCluster = 2;
+static int ordered_slices(const CnGemm &q)
+{
+    const int kb_total = (q.k + 63) >> 6;
+    int split = q.split_k;
+    if (split == 0) {
+        const int m_tiles = (q.m + kTileM - 1) / kTileM, bn = tile_n(q.n);
+        const long long tiles = (long long)((m_tiles + kOrderedCluster - 1) / kOrderedCluster) * ((q.n + bn - 1) / bn);
+        split = (int)(2.0 * kOrderedClusters / (double)tiles + 0.5);
+        if (split < 1) split = 1;
+    }
+    if (split > kb_total) split = kb_total;
+    const int per = (kb_total + split - 1) / split;
+    return (kb_total + per - 1) / per;                          // no empty slices
+}
+
+static size_t ordered_slice_floats(const CnGemm &q) { return (size_t)q.m * (size_t)((q.n + 7) & ~7); }
+
+// bytes of the partial-product workspace of an ordered launch (sum over its split problems of slices x m x n_pad x 4) and
+// optionally each problem's slice count; pure host code.  Returns NULL on success or a static error string.
+const char *gemm_bf16x3_ordered_workspace(const CnGemm *problems, int n_problems, size_t *bytes, int *slices)
+{
+    if (n_problems < 1 || n_problems > kMaxProblems) return "n_problems out of range";
+    size_t total = 0;
+    for (int i = 0; i < n_problems; ++i) {
+        const CnGemm &q = problems[i];
+        if (q.m < 1 || q.n < 1 || q.k < 1) return "m, n, k must be positive";
+        if (q.split_k < 0) return "split_k must be >= 0";
+        const int s = ordered_slices(q);
+        if (slices) slices[i] = s;
+        if (s > 1) total += (size_t)s * ordered_slice_floats(q) * sizeof(float);
+    }
+    *bytes = total;
+    return nullptr;
+}
+
 // optional device timing of every launch (bench.py's roofline): CUDA events on the launching stream, drained by
 // gemm_bf16x3_time_ms
 #include <vector>
@@ -440,11 +546,14 @@ float gemm_bf16x3_time_ms(int *launches, double *flops)
     return total;
 }
 
-// returns NULL on success or a static error string (called from c_abi.cu)
-const char *gemm_bf16x3_launch(const CnGemm *problems, int n_problems, cudaStream_t stream, int *items_out)
+// returns NULL on success or a static error string (called from c_abi.cu).  ordered: split problems take their slice count
+// from ordered_slices and store their partial tiles into `workspace` (gemm_bf16x3_ordered_workspace bytes, 32-byte aligned),
+// then splitk_reduce_kernel adds them to C in slice order.
+const char *gemm_bf16x3_launch(const CnGemm *problems, int n_problems, cudaStream_t stream, int *items_out, bool ordered,
+                               void *workspace, size_t workspace_bytes)
 {
     static int num_sms = 0;
-    static bool attr_set = false;
+    static bool attr_set[2] = {false, false};
     static int forced_cluster = -1;
     if (n_problems < 1 || n_problems > kMaxProblems) return "n_problems out of range";
     if (num_sms == 0) {
@@ -457,11 +566,23 @@ const char *gemm_bf16x3_launch(const CnGemm *problems, int n_problems, cudaStrea
         forced_cluster = env ? atoi(env) : 0;
         if (forced_cluster != 1 && forced_cluster != 2 && forced_cluster != 4) forced_cluster = 0;
     }
-    if (!attr_set) {
-        if (cudaFuncSetAttribute(gemm_bf16x3_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemLimit + 1024) != cudaSuccess)
-            return "cudaFuncSetAttribute(MaxDynamicSharedMemorySize) failed";
-        attr_set = true;
+    if (ordered) {
+        size_t need = 0;
+        if (const char *msg = gemm_bf16x3_ordered_workspace(problems, n_problems, &need, nullptr)) return msg;
+        if (need > 0 && !workspace) return "workspace is NULL";
+        if (need > 0 && (reinterpret_cast<uintptr_t>(workspace) & 31)) return "workspace must be 32-byte aligned";
+        if (workspace_bytes < need) return "workspace too small (see cn_gemm_bf16x3_ordered_workspace_bytes)";
     }
+    if (!attr_set[ordered]) {
+        if (cudaFuncSetAttribute(ordered ? gemm_bf16x3_kernel<true> : gemm_bf16x3_kernel<false>,
+                                 cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemLimit + 1024) != cudaSuccess)
+            return "cudaFuncSetAttribute(MaxDynamicSharedMemorySize) failed";
+        attr_set[ordered] = true;
+    }
+    static thread_local ReduceArgs red;
+    red.n_problems = 0;
+    red.total_units = 0;
+    float *ws_next = static_cast<float *>(workspace);
     static thread_local GemmArgs args;
     int max_b_bytes = 0;
     long long total_kb_items = 0;
@@ -474,11 +595,7 @@ const char *gemm_bf16x3_launch(const CnGemm *problems, int n_problems, cudaStrea
         if ((reinterpret_cast<uintptr_t>(q.a.hi) | reinterpret_cast<uintptr_t>(q.a.lo) | reinterpret_cast<uintptr_t>(q.b.hi) |
              reinterpret_cast<uintptr_t>(q.b.lo)) & 15) return "operand pointers must be 16-byte aligned";
         if (q.act < 0 || q.act > 2) return "unknown activation";
-        int bn = q.n <= 256 ? ((q.n + 15) & ~15) : 256;
-        if (q.n > 256) {       // even n-tiles (e.g. 320 -> 2 x 160) instead of a full tile and a sliver
-            const int tiles = (q.n + 255) / 256;
-            bn = (((q.n + tiles - 1) / tiles) + 15) & ~15;
-        }
+        const int bn = tile_n(q.n);
         g.bn = bn;
         g.m = q.m; g.n = q.n; g.k = q.k;
         g.m_tiles = (q.m + kTileM - 1) / kTileM;
@@ -490,9 +607,20 @@ const char *gemm_bf16x3_launch(const CnGemm *problems, int n_problems, cudaStrea
         int split = q.split_k;
         if (split < 0) return "split_k must be >= 0";
         if (split > kb_total) split = kb_total;
+        if (ordered) split = ordered_slices(q);
         g.split_k = split;                                   // 0 = decided below (auto), 1 = no split
-        g.mode = split == 1 ? (q.accumulate ? 1 : 0) : 2;
-        if (g.mode == 2 && (q.bias || q.act)) return "split-K products cannot carry a bias or an activation";
+        g.mode = split == 1 ? (q.accumulate ? 1 : 0) : ordered ? 3 : 2;
+        if (g.mode >= 2 && (q.bias || q.act)) return "split-K products cannot carry a bias or an activation";
+        if (g.mode == 3) {                                   // the kernel stores slice s at c + s * m * ldc
+            ReduceProblem &r = red.p[red.n_problems++];
+            r.c = q.c; r.ldc = q.ldc; r.p = ws_next;
+            r.m = q.m; r.n = q.n; r.n_pad = (q.n + 7) & ~7; r.slices = split;
+            r.vec = (q.ldc & 3) == 0 && (reinterpret_cast<uintptr_t>(q.c) & 15) == 0;
+            r.unit0 = red.total_units;
+            red.total_units += (long long)q.m * (r.n_pad >> 2);
+            g.c = ws_next; g.ldc = r.n_pad;
+            ws_next += (size_t)split * ordered_slice_floats(q);
+        }
         const int b_tile = g.b_mn ? ((bn + 63) / 64) * 8192 : bn * 128;
         g.stage_tx = (unsigned)(kABytes * (1 + g.a_lo_on) + b_tile * (1 + g.b_lo_on));
         if (b_tile > max_b_bytes) max_b_bytes = b_tile;
@@ -526,7 +654,7 @@ const char *gemm_bf16x3_launch(const CnGemm *problems, int n_problems, cudaStrea
             pa[0].val.clusterDim.x = (unsigned)cluster; pa[0].val.clusterDim.y = 1; pa[0].val.clusterDim.z = 1;
             probe.attrs = pa; probe.numAttrs = 1;
             int n = 0;
-            if (cudaOccupancyMaxActiveClusters(&n, gemm_bf16x3_kernel, &probe) != cudaSuccess || n < 1) n = num_sms / cluster;
+            if (cudaOccupancyMaxActiveClusters(&n, gemm_bf16x3_kernel<false>, &probe) != cudaSuccess || n < 1) n = num_sms / cluster;
             active[cluster] = n;
         }
         if (active[cluster] < max_clusters) max_clusters = active[cluster];
@@ -578,7 +706,13 @@ const char *gemm_bf16x3_launch(const CnGemm *problems, int n_problems, cudaStrea
         g_timer.pending.push_back(p);
         for (int i = 0; i < n_problems; ++i) g_timer.flops += 2.0 * problems[i].m * (double)problems[i].n * problems[i].k;
     }
-    const cudaError_t err = cudaLaunchKernelEx(&cfg, gemm_bf16x3_kernel, args);
+    cudaError_t err = ordered ? cudaLaunchKernelEx(&cfg, gemm_bf16x3_kernel<true>, args) : cudaLaunchKernelEx(&cfg, gemm_bf16x3_kernel<false>, args);
+    if (err == cudaSuccess && red.n_problems > 0) {
+        long long blocks = (red.total_units + 255) / 256;
+        if (blocks > 148 * 4) blocks = 148 * 4;
+        splitk_reduce_kernel<<<(unsigned)blocks, 256, 0, stream>>>(red);
+        err = cudaGetLastError();
+    }
     if (g_timer.enabled) cudaEventRecord(g_timer.pending.back().second, stream);
     if (items_out) *items_out = args.total_items;
     return err == cudaSuccess ? nullptr : cudaGetErrorString(err);

@@ -2,13 +2,20 @@
 the library's hand-written sm_100a kernels -- no cuBLAS product anywhere in `Policy.evaluate_actions` + `backward()`.
 
 * `gemm`               cn_gemm_bf16x3: TMA-fed tcgen05 split-bf16 3-pass GEMM (csrc/gemm_bf16x3.cu), K-major or MN-major
-                       operands, grouped problems, split-K with atomic accumulation for the weight gradients.
+                       operands, grouped problems, split-K with atomic accumulation for the weight gradients -- or, while
+                       `ordered()` holds, cn_gemm_bf16x3_ordered: the split-K partial products summed in a fixed order.
 * `linear`             y = act(x W^T + b) and its three backward products (dx = dy W, dW = dy^T x, db) on that kernel.
 * `EdgeGruSequence`    the two edge GRUs of the DS-RNN over a [T, n] rollout chunk (srnn_model.py:53-104, 201-215): forward =
                        T launches of the rollout's tcgen05 edge kernel in training mode (cn_dsrnn_edge_sequence_step: also
                        writes the gate values and the split-bf16 operands of the backward); backward = per step one gate
                        kernel (cn_gru_gates_backward_pairs) + one grouped recurrent product, then the input and weight
                        gradients of the whole sequence as three grouped GEMM launches.
+
+Reproducibility: the split-K weight gradients and the edge-encoder gradient combine partial sums from many CTAs.  By default
+they do so with atomics, whose order varies from run to run (results agree to ~1e-6 relative, not bit for bit).  While
+`ordered()` is true -- inside an update of `PPO(deterministic=True)` (training.cuda_deterministic), or whenever
+`torch.use_deterministic_algorithms(True)` is in effect -- they write their partial sums to a workspace taken from torch's
+caching allocator and add them in a fixed order instead, so the same inputs give the same gradients bit for bit.
 
 Everything here needs CUDA tensors on a B200; there is no CPU fallback (the CPU tests exercise the torch restatement in
 model.py, which is also the cross-check of these kernels on the GPU).
@@ -20,6 +27,14 @@ import torch
 from . import _lib, abi
 
 BF16 = torch.bfloat16
+
+# Set by PPO(deterministic=True) for the duration of its update (as PPO sets model.SEQUENCE_GEMM); see `ordered`.
+DETERMINISTIC = False
+
+
+def ordered():
+    """True when reductions over many CTAs must be summed in a fixed order (bit-reproducible) rather than with atomics."""
+    return DETERMINISTIC or torch.are_deterministic_algorithms_enabled()
 
 
 def _ptr(t):
@@ -74,10 +89,7 @@ def _operand(pair, mn_major):
     return abi.CnGemmOperand(_ptr(hi), _ptr(lo), ld, 1 if mn_major else 0, 0)
 
 
-def gemm(problems):
-    """Launch up to abi.GEMM_MAX_PROBLEMS products in one grouped tcgen05 kernel.  Each problem is a dict:
-    a=(hi, lo), a_mn=bool, b=(hi, lo), b_mn=bool, c=fp32 [m, n] (unit column stride), bias=None, act=0, accumulate=False,
-    split_k=1 (0 = library's choice; >1 / 0 add partial products to c atomically: c must be initialised)."""
+def _gemm_array(problems):
     if not 1 <= len(problems) <= abi.GEMM_MAX_PROBLEMS:
         raise ValueError("1..%d problems per launch" % abi.GEMM_MAX_PROBLEMS)
     arr = (abi.CnGemm * len(problems))()
@@ -98,9 +110,48 @@ def gemm(problems):
         g.c, g.ldc, g.bias = _ptr(c), (c.stride(0) if m > 1 else max(c.stride(0), n)), _ptr(bias)
         g.m, g.n, g.k = m, n, k
         g.act, g.accumulate, g.split_k = int(p.get("act", 0)), int(bool(p.get("accumulate", False))), int(p.get("split_k", 1))
+    return arr, keep, dev
+
+
+def ordered_workspace(problems):
+    """(bytes, slice count of each problem) of an ordered launch of `problems` (same dicts as `gemm`); host-side only."""
+    arr, _, _ = _gemm_array(problems)
+    need, slices = C.c_size_t(), (C.c_int * len(problems))()
+    _lib.check(_lib.load().cn_gemm_bf16x3_ordered_workspace_bytes(arr, len(problems), C.byref(need), slices),
+               "cn_gemm_bf16x3_ordered_workspace_bytes")
+    return need.value, list(slices)
+
+
+def gemm(problems):
+    """Launch up to abi.GEMM_MAX_PROBLEMS products in one grouped tcgen05 kernel.  Each problem is a dict:
+    a=(hi, lo), a_mn=bool, b=(hi, lo), b_mn=bool, c=fp32 [m, n] (unit column stride), bias=None, act=0, accumulate=False,
+    split_k=1 (0 = library's choice; >1 / 0 add partial products to c: c must be initialised).  While `ordered()` holds the
+    partial products are summed in slice order (cn_gemm_bf16x3_ordered, workspace from the caching allocator)."""
+    arr, keep, dev = _gemm_array(problems)
+    lib = _lib.load()
     with _on_device(dev):
-        _lib.check(_lib.load().cn_gemm_bf16x3(arr, len(problems), _stream(dev)), "cn_gemm_bf16x3")
+        if ordered():
+            need = C.c_size_t()
+            _lib.check(lib.cn_gemm_bf16x3_ordered_workspace_bytes(arr, len(problems), C.byref(need), None),
+                       "cn_gemm_bf16x3_ordered_workspace_bytes")
+            ws = torch.empty(need.value, dtype=torch.uint8, device=dev) if need.value else None
+            _lib.check(lib.cn_gemm_bf16x3_ordered(arr, len(problems), _ptr(ws), need.value, _stream(dev)), "cn_gemm_bf16x3_ordered")
+        else:
+            _lib.check(lib.cn_gemm_bf16x3(arr, len(problems), _stream(dev)), "cn_gemm_bf16x3")
     COUNTERS["gemm_launches"] += 1
+
+
+def encoder_grad(de, e_hi, ld_e, x, dw, db):
+    """dw [64, 2] += sum_rows [e > 0] de x^T, db [64] += sum_rows [e > 0] de (cn_encoder_grad; cn_encoder_grad_ordered while
+    `ordered()` holds).  de [rows, 64] fp32, e_hi the bf16 image of e with row stride ld_e, x [rows, 2]."""
+    lib, dev, rows = _lib.load(), de.device, x.shape[0]
+    with _on_device(dev):
+        if ordered():
+            ws = torch.empty(lib.cn_encoder_grad_ordered_workspace_bytes(rows), dtype=torch.uint8, device=dev)
+            _lib.check(lib.cn_encoder_grad_ordered(_ptr(de), _ptr(e_hi), ld_e, _ptr(x), _ptr(dw), _ptr(db), rows, _ptr(ws), ws.numel(),
+                                                   _stream(dev)), "cn_encoder_grad_ordered")
+        else:
+            _lib.check(lib.cn_encoder_grad(_ptr(de), _ptr(e_hi), ld_e, _ptr(x), _ptr(dw), _ptr(db), rows, _stream(dev)), "cn_encoder_grad")
 
 
 COUNTERS = {"gemm_launches": 0, "kernel_launches": 0}
@@ -289,7 +340,6 @@ class EdgeGruSequence(torch.autograd.Function):
             db_ih = torch.cat([colsum[256:768], colsum[:256]])
             db_hh = colsum[256:]
             dw_enc, db_enc = torch.zeros(64, 2, dtype=torch.float32, device=dev), torch.zeros(64, dtype=torch.float32, device=dev)
-            _lib.check(lib.cn_encoder_grad(_ptr(de[sl]), _ptr(e_hi[sl]), 72, _ptr(x), _ptr(dw_enc), _ptr(db_enc), x.shape[0], stream),
-                       "cn_encoder_grad")                                    # ReLU mask + the two reductions in one pass over de
+            encoder_grad(de[sl], e_hi[sl], 72, x, dw_enc, db_enc)            # ReLU mask + the two reductions in one pass over de
             grads.append((dw_enc, db_enc, unperm(dwx[k, :768, :64]), dwh[k], db_ih, db_hh))
         return (None, None, None, grad_h0, None) + grads[0] + grads[1]

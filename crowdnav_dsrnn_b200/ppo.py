@@ -12,6 +12,11 @@ Added for the sharded rollout (BASELINE.json configs[4]: envs sharded over 1/2/4
 * `max_envs_per_pass`: a minibatch is processed in sub-chunks of whole env trajectories with gradient accumulation
   (same gradient, bounded activation memory: T=30 steps x 21 edges x 768 gate columns per env are kept for backward).
 
+`deterministic=True` (the reference's training.cuda_deterministic) makes the native update bit-reproducible: its split-K
+weight gradients and edge-encoder gradient are summed in a fixed order instead of with atomics (native.ordered).  The
+other update paths are reproducible already.  With several ranks every rank runs the same ordered kernels; whether two
+multi-GPU runs then agree bit for bit also depends on the order of NCCL's all-reduce, which this does not control.
+
 The rollout forward (`Policy.act`) is the CUDA hot path.  The differentiable sequence forward used here is
 `Policy.evaluate_actions` (model.py): the recurrent units run as masked GRU sequences -- one autograd node each, cuBLAS
 GEMMs (fp32, `tf32=True`, or split-bf16 3-pass with `bf16x3=True`) around the library's hand-written gate kernels
@@ -46,7 +51,7 @@ def normalized_advantages(rollouts, group=None):
 class PPO:
     def __init__(self, actor_critic, clip_param, ppo_epoch, num_mini_batch, value_loss_coef, entropy_coef, lr=None, eps=None,
                  max_grad_norm=None, use_clipped_value_loss=True, group=None, max_envs_per_pass=None, tf32=False, bf16x3=False,
-                 native=False):
+                 native=False, deterministic=False):
         self.actor_critic = actor_critic
         self.clip_param = clip_param
         self.ppo_epoch = ppo_epoch
@@ -60,6 +65,7 @@ class PPO:
         self.tf32 = bool(tf32)         # TF32 tensor cores for the fp32 GEMMs of the update's forward + backward
         self.bf16x3 = bool(bf16x3)     # split-bf16 3-pass tensor-core GEMMs (fp32-level accuracy) for the recurrent products
         self.native = bool(native)     # every contraction of the update on the library's own tcgen05 kernels (native.py), CUDA only
+        self.deterministic = bool(deterministic)   # native path: reductions in a fixed order, same gradients bit for bit
         self.optimizer = optim.Adam(actor_critic.parameters(), lr=lr, eps=eps)
         self.perm_fn = None            # tests / reproducibility: callable(num_processes) -> env permutation
         self.allreduce_calls = 0
@@ -150,19 +156,23 @@ class PPO:
     def update(self, rollouts, sync=True):
         """`sync=False` returns the three averaged losses as a device tensor instead of Python floats (no host synchronisation)."""
         from . import model as _model
+        from . import native as _native
 
-        prev, prev_gemm = torch.backends.cuda.matmul.allow_tf32, _model.SEQUENCE_GEMM
+        prev, prev_gemm, prev_det = torch.backends.cuda.matmul.allow_tf32, _model.SEQUENCE_GEMM, _native.DETERMINISTIC
         prev_impl = getattr(self.actor_critic, "sequence_impl", "batched")
         torch.backends.cuda.matmul.allow_tf32 = prev or self.tf32
         if self.bf16x3:
             _model.SEQUENCE_GEMM = "bf16x3"
         if self.native and rollouts.device.type == "cuda":
             self.actor_critic.sequence_impl = "native"
+        if self.deterministic:
+            _native.DETERMINISTIC = True
         try:
             return self._update(rollouts, sync)
         finally:
             torch.backends.cuda.matmul.allow_tf32 = prev
             _model.SEQUENCE_GEMM = prev_gemm
+            _native.DETERMINISTIC = prev_det
             self.actor_critic.sequence_impl = prev_impl
 
     def _update(self, rollouts, sync=True):

@@ -6,6 +6,10 @@ device resident, no host synchronisation inside the rollout), `get_value` bootst
 `progress.csv` has the reference's columns (train.py:363-372).  Episode statistics are reduced on the device
 (the reference walks a Python list of info dicts per step, train.py:263-276).
 
+`training.cuda_deterministic` (the reference's switch: its train.py puts cuDNN into deterministic mode) makes a run
+reproducible: cuDNN is set to deterministic mode and the native update sums its split-K reductions in a fixed order
+(`PPO(deterministic=True)`), so two runs with the same seed write checkpoints with identical tensors.
+
 Under `torch.distributed` every rank runs this function with its own shard of `training.num_processes` envs
 (env ids offset by rank so the episode seeds do not collide) and `PPO` averages the gradients; rank 0 writes artefacts.
 """
@@ -79,6 +83,10 @@ def train(config, device=None, num_updates=None, output_dir=None, actor_critic=N
     device = torch.device(device if device is not None else "cuda:0")
     torch.manual_seed(config.env.seed + rank)
     torch.cuda.manual_seed_all(config.env.seed + rank)
+    deterministic = bool(getattr(config.training, "cuda_deterministic", False))
+    if deterministic:
+        torch.backends.cudnn.benchmark = False
+        torch.backends.cudnn.deterministic = True
     N, T, H = int(config.training.num_processes), int(config.ppo.num_steps), int(config.sim.human_num)
     envs = CrowdVecEnv(config, N, device, seed=config.env.seed, phase="train", env_id_offset=rank * N, nenv=N * world)
     if actor_critic is None:
@@ -95,7 +103,7 @@ def train(config, device=None, num_updates=None, output_dir=None, actor_critic=N
     agent = PPO(actor_critic, config.ppo.clip_param, config.ppo.epoch, config.ppo.num_mini_batch, config.ppo.value_loss_coef,
                 config.ppo.entropy_coef, lr=config.training.lr, eps=config.training.eps,
                 max_grad_norm=config.training.max_grad_norm, max_envs_per_pass=max_envs_per_pass, tf32=tf32_update, bf16x3=bf16x3_update,
-                native=native_update)
+                native=native_update, deterministic=deterministic)
     obs = envs.reset()
     for k in rollouts.obs:
         rollouts.obs[k][0].copy_(obs[k])
@@ -184,7 +192,8 @@ def train(config, device=None, num_updates=None, output_dir=None, actor_critic=N
 
 
 def main(argv=None):
-    """`python -m crowdnav_dsrnn_b200.train [--output_dir DIR] [--num_updates K] [--envs N] [--humans H] [--native]`:
+    """`python -m crowdnav_dsrnn_b200.train [--output_dir DIR] [--num_updates K] [--envs N] [--humans H] [--native]
+    [--deterministic]`:
     the reference's `python train.py` on the batched backend (its settings come from the config file; here the ones that
     matter for a batch of thousands of envs can be given on the command line)."""
     import argparse
@@ -199,8 +208,12 @@ def main(argv=None):
     ap.add_argument("--kinematics", default="holonomic", choices=["holonomic", "unicycle"])
     ap.add_argument("--envs_per_pass", type=int, default=4096)
     ap.add_argument("--native", action="store_true", help="PPO update on the library's own tensor-core kernels")
+    ap.add_argument("--deterministic", action="store_true",
+                    help="training.cuda_deterministic: the same seed gives the same checkpoints (ordered reductions in the update)")
     args = ap.parse_args(argv)
     cfg = Config(kinematics=args.kinematics, human_num=args.humans)
+    if args.deterministic:
+        cfg.training.cuda_deterministic = True
     if args.envs:
         cfg.training.num_processes = args.envs
     if args.output_dir:

@@ -345,11 +345,19 @@ int cn_attention_train_backward(const float *o, const float *qt, const float *al
 
 /* Gradient of the edge encoder e = ReLU(W_enc x + b), x [rows, 2] (srnn_model.py:201-215): from de = dL/de [rows, 64] (fp32) and
  * the sign of e (bf16 image with row stride ld_e):  dw[64, 2] += sum_rows [e > 0] de x^T,  db[64] += sum_rows [e > 0] de.
- * dw / db must hold the initial value (zeros).  One HBM-bound pass over de. */
+ * dw / db must hold the initial value (zeros).  One HBM-bound pass over de.  cn_encoder_grad combines its block sums with
+ * atomics (the order of the additions varies from run to run); cn_encoder_grad_ordered writes them to `workspace`
+ * (cn_encoder_grad_ordered_workspace_bytes(rows) bytes, 16-byte aligned, owned by the caller) and adds them to dw / db in a
+ * fixed order: the same inputs give the same bits.  A NULL, misaligned or too small workspace is refused. */
 int cn_encoder_grad(const float *de, const void *e_hi, int ld_e, const float *x, float *dw, float *db, long long rows, void *stream);
+size_t cn_encoder_grad_ordered_workspace_bytes(long long rows);
+int cn_encoder_grad_ordered(const float *de, const void *e_hi, int ld_e, const float *x, float *dw, float *db, long long rows,
+                            void *workspace, size_t workspace_bytes, void *stream);
 
 /* Generic split-bf16 3-pass tensor-core GEMM (tcgen05, TMA-fed, fp32 accumulation in TMEM):
- *   C[m, n] (=, +=, or atomically += for split-K)  (A_hi + A_lo)(B_hi + B_lo) minus the lo*lo term  (+ bias[n], activation).
+ *   C[m, n] (=, +=, or += for split-K)  (A_hi + A_lo)(B_hi + B_lo) minus the lo*lo term  (+ bias[n], activation).
+ * Split-K partial products are added to C atomically by cn_gemm_bf16x3 (the order of the additions varies from run to run)
+ * and in slice order by cn_gemm_bf16x3_ordered (below).
  * An operand is K-major (row-major [m|n, k] array) or MN-major (row-major [k, m|n] array); lo == NULL drops that operand's
  * correction pass.  Up to CN_GEMM_MAX_PROBLEMS independent problems per launch (grouped GEMM). */
 #define CN_GEMM_MAX_PROBLEMS 4
@@ -368,9 +376,19 @@ typedef struct CnGemm {
     int act;               /* 0 none, 1 ReLU, 2 tanh */
     int accumulate;        /* split_k == 1 only: C += product instead of C = product */
     int split_k;           /* 1: no split.  >1 or 0 (= chosen by the library): k is cut into slices whose partial products are added
-                              to C with atomics -- C must hold the initial value (zeros); no bias / activation */
+                              to C -- C must hold the initial value (zeros); no bias / activation */
 } CnGemm;
 int cn_gemm_bf16x3(const CnGemm *problems, int n_problems, void *stream);
+/* Bit-reproducible form of cn_gemm_bf16x3: each k-slice stores its partial product into its own slice of `workspace` (owned by
+ * the caller, 32-byte aligned), then C = C_in + P_0 + P_1 + ... + P_{S-1} is summed in slice order.  The slice count S of a
+ * problem is a function of its own (m, n, k, split_k) only: split_k > 1 is taken as given (capped at one slice per 64-deep
+ * k-block), split_k = 0 evaluates the library's automatic choice for the problem alone on a 148-SM budget.  So a problem
+ * gives the same bits launched alone or grouped, on any device.  Problems with S = 1 are stored / accumulated directly.
+ * cn_gemm_bf16x3_ordered_workspace_bytes returns the bytes the launch needs (sum over the problems with S > 1 of
+ * S * m * n8 * 4, n8 = n rounded up to 8; pure host code) and, when `slices` is not NULL, each problem's S.  A launch whose
+ * workspace is NULL, misaligned or smaller than that is refused (nothing is launched); no workspace is needed when it is 0. */
+int cn_gemm_bf16x3_ordered_workspace_bytes(const CnGemm *problems, int n_problems, size_t *bytes, int *slices);
+int cn_gemm_bf16x3_ordered(const CnGemm *problems, int n_problems, void *workspace, size_t workspace_bytes, void *stream);
 /* Optional device timing of every cn_gemm_bf16x3 launch of this process (bench.py's roofline): CUDA events on the launching
  * stream; cn_gemm_time_ms synchronises them and returns the accumulated milliseconds, launch count and algorithmic FLOPs
  * (2 m n k per problem) since the last call, and resets them. */
