@@ -10,6 +10,11 @@ device resident, no host synchronisation inside the rollout), `get_value` bootst
 reproducible: cuDNN is set to deterministic mode and the native update sums its split-K reductions in a fixed order
 (`PPO(deterministic=True)`), so two runs with the same seed write checkpoints with identical tensors.
 
+`training.save_train_state` (`--save-state`) also writes training-state files next to the checkpoints (train_state.py),
+and `training.resume` with `training.load_path` (`--resume PATH`) continues a run from one: in deterministic mode the
+continued run writes the same checkpoints as a run that was never interrupted.  `load_path` may also name a plain
+`state_dict` (a `%.5i.pt` checkpoint or a shipped one): its weights start a fresh run.
+
 Under `torch.distributed` every rank runs this function with its own shard of `training.num_processes` envs
 (env ids offset by rank so the episode seeds do not collide) and `PPO` averages the gradients; rank 0 writes artefacts.
 """
@@ -25,6 +30,7 @@ import torch
 import torch.distributed as dist
 
 from . import abi
+from . import train_state
 from .envs import CrowdVecEnv
 from .model import Policy
 from .ppo import PPO, update_linear_schedule
@@ -77,21 +83,53 @@ def _tensorboard_writer(out_dir):
     return SummaryWriter(log_dir=os.path.join(out_dir, "events"))
 
 
+def _resume_source(config, n_envs, world, rank, deterministic):
+    """What `training.load_path` holds when `training.resume` is set: None (no resume), ("weights", state_dict, None) or
+    ("state", shared, shard) of a training-state file that this run can continue (else TrainStateMismatch)."""
+    if not getattr(config.training, "resume", False):
+        return None
+    path = getattr(config.training, "load_path", None)
+    if not path:
+        raise ValueError("training.resume is set but training.load_path names no file to resume from")
+    source = train_state.load(path, rank)
+    if source[0] == "state":
+        train_state.check_keys(source[1]["keys"], train_state.run_keys(config, n_envs, world, deterministic))
+    return source
+
+
+def _drop_progress_after(path, last):
+    """A resumed run appends to progress.csv: rows the interrupted run wrote after the update it resumes from go first."""
+    if not os.path.exists(path):
+        return
+    with open(path, newline="") as f:
+        rows = list(csv.reader(f))
+    keep = rows[:1] + [r for r in rows[1:] if r and int(r[0]) <= last]
+    if len(keep) != len(rows):
+        with open(path, "w", newline="") as f:
+            csv.writer(f).writerows(keep)
+
+
 def train(config, device=None, num_updates=None, output_dir=None, actor_critic=None, log=print, max_envs_per_pass=None,
           keep_hidden_history=False, tf32_update=False, bf16x3_update=False, native_update=False):
     rank, world = _rank_world()
     device = torch.device(device if device is not None else "cuda:0")
+    deterministic = bool(getattr(config.training, "cuda_deterministic", False))
+    N, T, H = int(config.training.num_processes), int(config.ppo.num_steps), int(config.sim.human_num)
+    resume = _resume_source(config, N, world, rank, deterministic)        # refused here, before any GPU work
+    save_state = bool(getattr(config.training, "save_train_state", False))
+    state_keys = train_state.run_keys(config, N, world, deterministic) if save_state else None
     torch.manual_seed(config.env.seed + rank)
     torch.cuda.manual_seed_all(config.env.seed + rank)
-    deterministic = bool(getattr(config.training, "cuda_deterministic", False))
     if deterministic:
         torch.backends.cudnn.benchmark = False
         torch.backends.cudnn.deterministic = True
-    N, T, H = int(config.training.num_processes), int(config.ppo.num_steps), int(config.sim.human_num)
     envs = CrowdVecEnv(config, N, device, seed=config.env.seed, phase="train", env_id_offset=rank * N, nenv=N * world)
     if actor_critic is None:
         actor_critic = Policy(envs.observation_space.spaces, envs.action_space, base=config.robot.policy, base_kwargs=config)
     actor_critic.to(device)
+    if resume is not None and resume[0] == "weights":
+        actor_critic.load_state_dict(resume[1])
+        actor_critic.invalidate_weights()
     if world > 1:                         # same initial weights everywhere
         with torch.no_grad():             # in place on the parameter itself: bumps its version, so packed copies are refreshed
             for p in actor_critic.parameters():
@@ -107,6 +145,11 @@ def train(config, device=None, num_updates=None, output_dir=None, actor_critic=N
     obs = envs.reset()
     for k in rollouts.obs:
         rollouts.obs[k][0].copy_(obs[k])
+    first = 0
+    if resume is not None and resume[0] == "state":
+        train_state.restore(resume[1], resume[2], actor_critic, agent.optimizer, envs.engine, rollouts, device)
+        first = resume[1]["update"] + 1
+    # num_updates counts from the start of the run: a resumed run goes on with update `first` up to the same end
     total_updates = int(config.training.num_env_steps) // T // (N * world)
     if num_updates is None:
         num_updates = total_updates
@@ -116,6 +159,8 @@ def train(config, device=None, num_updates=None, output_dir=None, actor_critic=N
         os.makedirs(os.path.join(out_dir, "checkpoints"), exist_ok=True)
         file_log = write_run_artefacts(config, out_dir)
         tboard = _tensorboard_writer(out_dir)
+        if first:
+            _drop_progress_after(os.path.join(out_dir, "progress.csv"), first - 1)
     # device-side episode statistics: [success, collision, timeout, episodes, return sum], reduced ONCE per update from the
     # per-step event / done / episode-return records (three small copies per step instead of ~20 reduction launches)
     stats = torch.zeros(5, dtype=torch.float64, device=device)
@@ -124,7 +169,7 @@ def train(config, device=None, num_updates=None, output_dir=None, actor_critic=N
     ret_rec = torch.zeros(T, N, dtype=torch.float32, device=device)
     history = []
     start = time.time()
-    for j in range(num_updates):
+    for j in range(first, num_updates):
         if config.training.use_linear_lr_decay:
             update_linear_schedule(agent.optimizer, j, max(total_updates, num_updates), config.training.lr)
         stats.zero_()
@@ -150,7 +195,8 @@ def train(config, device=None, num_updates=None, output_dir=None, actor_critic=N
             dist.all_reduce(stats)
         s = stats.tolist()
         total_steps = (j + 1) * N * world * T
-        row = {"misc/nupdates": j, "misc/total_timesteps": total_steps, "fps": int(total_steps / (time.time() - start)),
+        fps = int((total_steps - first * N * world * T) / (time.time() - start))       # steps of this process only
+        row = {"misc/nupdates": j, "misc/total_timesteps": total_steps, "fps": fps,
                "eprewmean": s[4] / s[3] if s[3] else float("nan"), "loss/policy_entropy": entropy,
                "loss/policy_loss": action_loss, "loss/value_loss": value_loss,
                "success": s[0] / s[3] if s[3] else float("nan"), "collision": s[1] / s[3] if s[3] else float("nan"),
@@ -167,6 +213,9 @@ def train(config, device=None, num_updates=None, output_dir=None, actor_critic=N
                     if fresh:
                         w.writeheader()
                     w.writerow(row)
+        if save_state and out_dir and (j % config.training.save_interval == 0 or j == num_updates - 1):
+            train_state.save(os.path.join(out_dir, "checkpoints"), j, total_steps, state_keys, actor_critic, agent.optimizer,
+                             envs.engine, rollouts, device, rank, world)
         if rank == 0 and j % config.training.log_interval == 0:
             msg = ("Updates %d, num timesteps %d, FPS %d, episodes %d: mean reward %.3f, success %.3f, collision %.3f, timeout %.3f, "
                    "entropy %.4f, value loss %.4f, policy loss %.5f" % (j, total_steps, row["fps"], row["episodes"], row["eprewmean"],
@@ -193,7 +242,7 @@ def train(config, device=None, num_updates=None, output_dir=None, actor_critic=N
 
 def main(argv=None):
     """`python -m crowdnav_dsrnn_b200.train [--output_dir DIR] [--num_updates K] [--envs N] [--humans H] [--native]
-    [--deterministic]`:
+    [--deterministic] [--save-state] [--resume PATH]`:
     the reference's `python train.py` on the batched backend (its settings come from the config file; here the ones that
     matter for a batch of thousands of envs can be given on the command line)."""
     import argparse
@@ -210,10 +259,20 @@ def main(argv=None):
     ap.add_argument("--native", action="store_true", help="PPO update on the library's own tensor-core kernels")
     ap.add_argument("--deterministic", action="store_true",
                     help="training.cuda_deterministic: the same seed gives the same checkpoints (ordered reductions in the update)")
+    ap.add_argument("--save-state", dest="save_state", action="store_true",
+                    help="training.save_train_state: write training-state files (%%.5i.state.pt) next to the checkpoints")
+    ap.add_argument("--resume", default=None, metavar="PATH",
+                    help="training.resume from training.load_path = PATH: a training-state file continues that run, a "
+                         "state_dict starts a fresh run from its weights")
     args = ap.parse_args(argv)
     cfg = Config(kinematics=args.kinematics, human_num=args.humans)
     if args.deterministic:
         cfg.training.cuda_deterministic = True
+    if args.save_state:
+        cfg.training.save_train_state = True
+    if args.resume:
+        cfg.training.resume = True
+        cfg.training.load_path = args.resume
     if args.envs:
         cfg.training.num_processes = args.envs
     if args.output_dir:
