@@ -32,6 +32,12 @@ INFO_COLUMNS = {
 }
 PREC_FP32, PREC_BF16X3, PREC_BF16, PREC_FP16 = 0, 1, 2, 3
 PRECISIONS = {"fp32": PREC_FP32, "bf16x3": PREC_BF16X3, "bf16": PREC_BF16, "fp16": PREC_FP16}
+# cn_env_render: palette (0xRRGGBB), marker sizes (metres / radians) and the accepted frame sizes (CN_RENDER_*)
+RENDER_RGB = {"background": 0xFFFFFF, "fov": 0xDCE9F7, "goal": 0xD62728, "human_in": 0x2CA02C, "human_out": 0x9E9E9E,
+              "robot": 0xFFC20E, "heading": 0x8C5A00, "invalid": 0xFF00FF}
+RENDER_GOAL_RADIUS = 0.15
+RENDER_HEADING_HALF = 0.5
+RENDER_MIN_SIZE, RENDER_MAX_SIZE, RENDER_SIZE_MULTIPLE = 32, 2048, 16
 
 
 class CnConfig(C.Structure):

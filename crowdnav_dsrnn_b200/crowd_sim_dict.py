@@ -8,6 +8,7 @@ import torch
 
 from .engine import CrowdEngine
 from .envs import LazyInfos
+from .render import check_mode, check_size
 from .spaces import crowd_spaces
 
 
@@ -78,6 +79,12 @@ class CrowdSimDict(object):
             st["counters"][:, 2] = int(test_case)
             eng.set_state(counters=st["counters"])
         return self._host_obs(eng.reset())
+
+    def render(self, mode="human", size=256):
+        """The env's frame as numpy uint8 [size, size, 3] (mode="rgb_array" only; drawn on the GPU)."""
+        check_mode(mode)
+        check_size(size)
+        return self._ensure().render(size=size)[0].cpu().numpy()
 
     def step(self, action, update=True):
         eng = self._ensure()

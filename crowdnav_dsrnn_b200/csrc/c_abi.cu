@@ -280,6 +280,32 @@ extern "C" int cn_env_observe(CnEnv *env, const CnObsOut *obs, void *stream)
     return CN_OK;
 }
 
+extern "C" int cn_launch_render(const EnvParams *P, const int32_t *ids, int k, const uint32_t *vis, int size, uint8_t *rgb,
+                                cudaStream_t stream);
+
+extern "C" int cn_env_render(CnEnv *env, const int32_t *env_ids_dev, int k, const uint32_t *visible_mask_dev, int size,
+                             uint8_t *rgb_dev, void *stream)
+{
+    if (!env) return fail(CN_ERR_ARG, "env is NULL");
+    if (size < CN_RENDER_MIN_SIZE || size > CN_RENDER_MAX_SIZE || size % CN_RENDER_SIZE_MULTIPLE != 0)
+        return fail(CN_ERR_ARG, "cn_env_render: size %d must be a multiple of %d in %d..%d", size, CN_RENDER_SIZE_MULTIPLE,
+                    CN_RENDER_MIN_SIZE, CN_RENDER_MAX_SIZE);
+    if (k < 0) return fail(CN_ERR_ARG, "cn_env_render: k %d < 0", k);
+    if (k == 0) {                                       // nothing to draw, nothing launched
+        env->last_launches = 0;
+        return CN_OK;
+    }
+    if (!rgb_dev) return fail(CN_ERR_ARG, "cn_env_render: rgb_dev is NULL");
+    if (((uintptr_t)rgb_dev & 15) != 0) return fail(CN_ERR_ARG, "cn_env_render: rgb_dev must be 16-byte aligned");
+    if (env_ids_dev == nullptr && k > env->p.n_envs)
+        return fail(CN_ERR_ARG, "cn_env_render: k %d > %d envs without an id list", k, env->p.n_envs);
+    CN_ON_DEVICE(env->device);
+    // no join_refill: the render reads only the running episodes' arrays, which the refill never writes (render.cu)
+    CN_CUDA((cudaError_t)cn_launch_render(&env->p, env_ids_dev, k, visible_mask_dev, size, rgb_dev, (cudaStream_t)stream));
+    env->last_launches = 1;
+    return CN_OK;
+}
+
 static int convert(CnEnv *env, const CnStateView *view, int dir, void *stream)
 {
     if (!env || !view) return fail(CN_ERR_ARG, "env/view is NULL");

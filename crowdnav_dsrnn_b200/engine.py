@@ -13,6 +13,7 @@ import ctypes as C
 import torch
 
 from . import _lib, abi
+from .render import check_size as _check_render_size
 
 
 def _ptr(t):
@@ -170,6 +171,32 @@ class CrowdEngine:
         _lib.check(self.lib.cn_env_observe(self.handle, C.byref(b.obs_struct), self._stream()), "cn_env_observe")
         self.launches += self.lib.cn_env_last_launches(self.handle)
         return b
+
+    def render(self, env_ids=None, size=256, out=None):
+        """rgb_array frames of envs `env_ids` (None: all; a list, or an int32 device tensor for a capturable call) drawn by
+        cn_env_render from the running state and the current buffer's visible_mask -> device uint8 [k, size, size, 3].
+        `out` (contiguous uint8 [k, size, size, 3] on this device) gives the frames a static address (CUDA graphs; a captured
+        render reads the visible_mask of the step buffer that was current at capture).  An id outside [0, N) gives a frame
+        of the "invalid" colour."""
+        size = _check_render_size(size)
+        dev = torch.device("cuda", self.device_index)
+        if env_ids is None:
+            ids, k = None, self.n
+        else:
+            ids = env_ids
+            if not (torch.is_tensor(ids) and ids.device == dev and ids.dtype == torch.int32 and ids.is_contiguous()):
+                ids = torch.as_tensor(env_ids, dtype=torch.int32).to(dev).contiguous()   # allocates: not capturable
+            ids = ids.reshape(-1)
+            k = ids.numel()
+        if out is None:
+            out = torch.empty(k, size, size, 3, dtype=torch.uint8, device=dev)
+        elif (out.dtype != torch.uint8 or out.device != dev or tuple(out.shape) != (k, size, size, 3)
+              or not out.is_contiguous()):
+            raise ValueError("out must be a contiguous uint8 tensor [%d, %d, %d, 3] on %s" % (k, size, size, dev))
+        _lib.check(self.lib.cn_env_render(self.handle, _ptr(ids), k, _ptr(self.bufs[self.cur].visible_mask), size,
+                                          _ptr(out), self._stream()), "cn_env_render")
+        self.launches += self.lib.cn_env_last_launches(self.handle)
+        return out
 
     # ------------------------------------------------------------------ state injection / extraction
     def _state_tensors(self):

@@ -8,7 +8,7 @@ Returned object (`CrowdVecEnv`):
   .observation_space.spaces / .action_space / .num_envs
   .reset()            -> dict[str, float32 Tensor on device]
   .step(action[N,2])  -> (obs dict, reward CPU float32 Tensor [N,1], done numpy bool [N], infos)
-  .step_async / .step_wait / .render / .close
+  .step_async / .step_wait / .render(mode="rgb_array") / .get_images / .close
   .venv.envs[0].env   -> object with .global_time .time_step .time_limit .robot.{time_step,v_pref} (evaluation.py:71)
 `infos` is a lazy sequence: `infos[i]` builds the reference-shaped dict
 ({"info": {..., "event": Collision()}, "episode": {"r","l","t"}}) only when it
@@ -24,6 +24,7 @@ import torch
 from . import abi
 from .engine import CrowdEngine, StepBuffers
 from .info import make_event
+from .render import check_mode, check_size, tile_images
 from .spaces import crowd_spaces
 
 
@@ -105,8 +106,10 @@ class _EnvView(object):
             t += self.time_step
         return t
 
-    def render(self, mode="human"):
-        raise NotImplementedError("rendering is out of scope (SURVEY section 2 row 2)")
+    def render(self, mode="human", size=256):
+        """This env's frame: numpy uint8 [size, size, 3] (mode="rgb_array" only)."""
+        check_mode(mode)
+        return self._vec.get_images([self._i], size=size)[0].cpu().numpy()
 
 
 class CrowdVecEnv(object):
@@ -166,8 +169,17 @@ class CrowdVecEnv(object):
         buf = self.engine.step(actions, auto_reset=True)
         return buf.obs(), buf.reward, buf.done, buf
 
-    def render(self, mode="human"):
-        raise NotImplementedError("rendering is out of scope (SURVEY section 2 row 2)")
+    def get_images(self, env_ids=None, size=256):
+        """baselines' VecEnv.get_images, kept on the device: uint8 [k, size, size, 3] of envs `env_ids` (default all),
+        drawn by the GPU from the running state (CrowdEngine.render)."""
+        return self.engine.render(env_ids, size=size)
+
+    def render(self, mode="human", size=256):
+        """baselines' VecEnv.render(mode="rgb_array"): the frames of the envs in `self.envs` (the first min(N, 64)) as one
+        numpy [rows * size, cols * size, 3] tile (tile_images layout).  Only "rgb_array" is supported."""
+        check_mode(mode)
+        check_size(size)
+        return tile_images(self.get_images(list(range(len(self.envs))), size=size).cpu().numpy())
 
     def close(self):
         self.engine.close()

@@ -199,6 +199,33 @@ int cn_env_get_state(CnEnv *env, const CnStateView *view, void *stream);
 int cn_env_observe(CnEnv *env, const CnObsOut *obs, void *stream);
 
 /*
+ * Frames (render(mode="rgb_array"), crowd_sim.py:1207-1461 without matplotlib): the square [-L/2, L/2]^2 of
+ * L = sim.square_width, row 0 at the top (+y up), pixel (i, j) sampled at its centre.  Layers, later over earlier:
+ * background; the robot's FOV wedge (robot.FOV < 2 only); the robot's goal disc; the humans as discs of their own radius
+ * in index order, coloured by bit i of visible_mask (all "inside" without a mask); the robot disc with a darker sector
+ * around its heading.  Colours are 0xRRGGBB, sizes in metres / radians.
+ */
+#define CN_RENDER_RGB_BACKGROUND  0xFFFFFF
+#define CN_RENDER_RGB_FOV         0xDCE9F7 /* wedge of the robot's field of view */
+#define CN_RENDER_RGB_GOAL        0xD62728
+#define CN_RENDER_RGB_HUMAN_IN    0x2CA02C /* human inside the robot's FOV (visible_mask bit set) */
+#define CN_RENDER_RGB_HUMAN_OUT   0x9E9E9E /* human outside the robot's FOV */
+#define CN_RENDER_RGB_ROBOT       0xFFC20E
+#define CN_RENDER_RGB_HEADING     0x8C5A00 /* sector of the robot disc around its heading */
+#define CN_RENDER_RGB_INVALID     0xFF00FF /* whole frame of an env id outside [0, n_envs) */
+#define CN_RENDER_GOAL_RADIUS     0.15     /* metres */
+#define CN_RENDER_HEADING_HALF    0.5      /* half-angle of the heading sector, radians */
+#define CN_RENDER_MIN_SIZE        32
+#define CN_RENDER_MAX_SIZE        2048
+#define CN_RENDER_SIZE_MULTIPLE   16
+/* frames of k envs (env_ids_dev [k] int32, NULL = envs 0..k-1) into rgb_dev [k, size, size, 3] uint8;
+ * visible_mask_dev [N] (may be NULL); 32 <= size <= 2048, size % 16 == 0.  An id outside [0, N) gives a frame of
+ * CN_RENDER_RGB_INVALID.  Reads only the running episodes' state: no allocation, no synchronisation (graph-capturable);
+ * k == 0 launches nothing. */
+int cn_env_render(CnEnv *env, const int32_t *env_ids_dev, int k, const uint32_t *visible_mask_dev, int size,
+                  uint8_t *rgb_dev, void *stream);
+
+/*
  * DS-RNN policy forward (SRNN.forward infer=True + DiagGaussian.fc_mean,
  * srnn_model.py:409-504, distributions.py:85-94).  Weights are DEVICE float32
  * tensors in the reference's own state_dict layout (row-major [out, in]).
