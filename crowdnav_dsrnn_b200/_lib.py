@@ -28,6 +28,7 @@ SYMBOLS = {
     "cn_env_get_state": (C.c_int, [_P, C.POINTER(abi.CnStateView), _P]),
     "cn_env_observe": (C.c_int, [_P, C.POINTER(abi.CnObsOut), _P]),
     "cn_env_render": (C.c_int, [_P, _P, C.c_int, _P, C.c_int, _P, _P]),
+    "cn_env_robot_act": (C.c_int, [_P, C.c_int32, _P, _P]),
     "cn_env_join": (C.c_int, [_P, _P]),
     "cn_env_refill": (C.c_int, [_P, _P]),
     "cn_dsrnn_set_refill_env": (C.c_int, [_P, _P]),

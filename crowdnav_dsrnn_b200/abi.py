@@ -18,6 +18,8 @@ INFO_DIM = 12
 HOLONOMIC, UNICYCLE = 0, 1
 POLICY_ORCA, POLICY_SOCIAL_FORCE = 0, 1
 HUMAN_POLICIES = {"orca": POLICY_ORCA, "social_force": POLICY_SOCIAL_FORCE}
+# model-based robots (robot.policy, policy_factory.py:12-17): their action comes from cn_env_robot_act
+ROBOT_POLICIES = {"orca": POLICY_ORCA, "social_force": POLICY_SOCIAL_FORCE}
 PHASE_TRAIN, PHASE_VAL, PHASE_TEST = 0, 1, 2
 PHASES = {"train": PHASE_TRAIN, "val": PHASE_VAL, "test": PHASE_TEST}
 EV_NOTHING, EV_DANGER, EV_REACH_GOAL, EV_COLLISION, EV_TIMEOUT = 0, 1, 2, 3, 4
@@ -188,6 +190,20 @@ def step_tables(time_step, time_limit):
     if timeout_step is None:
         raise ValueError("episode longer than %d steps is not supported" % (32 * STEP_TABLE_WORDS))
     return timeout_step, words
+
+
+def robot_policy_of(config):
+    """The CN_POLICY_* of a model-based robot (robot.policy = 'orca' / 'social_force'), None for the learned 'srnn' robot.
+    Raises NotImplementedError for any other name, and for a model-based robot with unicycle kinematics."""
+    name = config.robot.policy
+    if name == "srnn":
+        return None
+    if name not in ROBOT_POLICIES:
+        raise NotImplementedError("robot.policy=%r (the vectorised env runs 'srnn', 'orca' and 'social_force')" % (name,))
+    if config.action_space.kinematics != "holonomic":
+        raise NotImplementedError("robot.policy=%r outputs velocities: it needs action_space.kinematics='holonomic', not %r"
+                                  % (name, config.action_space.kinematics))
+    return ROBOT_POLICIES[name]
 
 
 def flatten_config(config, n_envs, phase=None, seed=None, env_id_offset=0, nenv=None,

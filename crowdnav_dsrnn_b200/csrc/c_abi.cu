@@ -280,6 +280,25 @@ extern "C" int cn_env_observe(CnEnv *env, const CnObsOut *obs, void *stream)
     return CN_OK;
 }
 
+extern "C" int cn_launch_robot_act(const EnvParams *P, int policy, float *action, cudaStream_t stream);
+
+extern "C" int cn_env_robot_act(CnEnv *env, int32_t policy, float *action_dev, void *stream)
+{
+    if (!env) return fail(CN_ERR_ARG, "env is NULL");
+    if (env->p.cfg.kinematics != CN_HOLONOMIC)
+        return fail(CN_ERR_ARG, "cn_env_robot_act: ORCA and social force output velocities; a unicycle robot cannot take them");
+    if (policy != CN_POLICY_ORCA && policy != CN_POLICY_SOCIAL_FORCE)
+        return fail(CN_ERR_ARG, "cn_env_robot_act: unknown policy %d (CN_POLICY_ORCA or CN_POLICY_SOCIAL_FORCE)", (int)policy);
+    if (!action_dev) return fail(CN_ERR_ARG, "cn_env_robot_act: action_dev is NULL");
+    if (((uintptr_t)action_dev & 7) != 0) return fail(CN_ERR_ARG, "cn_env_robot_act: action_dev must be 8-byte aligned");
+    CN_ON_DEVICE(env->device);
+    int rc = join_refill(env, (cudaStream_t)stream);
+    if (rc != CN_OK) return rc;
+    CN_CUDA((cudaError_t)cn_launch_robot_act(&env->p, policy, action_dev, (cudaStream_t)stream));
+    env->last_launches = 1;
+    return CN_OK;
+}
+
 extern "C" int cn_launch_render(const EnvParams *P, const int32_t *ids, int k, const uint32_t *vis, int size, uint8_t *rgb,
                                 cudaStream_t stream);
 

@@ -164,28 +164,42 @@ __device__ __forceinline__ float2 preferred_velocity(float4 pv, float4 gr)
     return make_float2((float)(gsp > 1.0 ? gdx / gsp : gdx), (float)(gsp > 1.0 ? gdy / gsp : gdy));
 }
 
-// One human's action by one G-lane group: the ORCA solve, or (kOpt builds only) the social-force step.
-// s_pv/s_gr/s_th: this env's humans (pre-step).  kOpt compiles the optional behaviours of SURVEY 8(f) N4 in
-// (humans.policy = social_force, random_policy_changing, random_unobservability); the default kernel has none of them.
-template <int G, bool kOpt>
+// Who solves, and where its neighbours come from: human i of the env staged in shared memory (the step kernel), or the
+// robot with the env's belief rows last_human_states as its neighbours (robot_act_kernel, robot.policy = orca /
+// social_force).  Every branch on it is a compile-time constant, so each form compiles to its own straight code.
+enum { AGENT_HUMAN = 0, AGENT_ROBOT_ORCA = 1, AGENT_ROBOT_SF = 2 };
+
+// One agent's action by one G-lane group: the ORCA solve, or (kOpt builds and the social-force robot only) the
+// social-force step.  kAgent == AGENT_HUMAN: s_pv/s_gr/s_th hold this env's humans (pre-step), i is the solver.  A robot
+// agent is rob_pv / P.a.rob_gr[e] and lane k reads belief row k of env e (i, s_pv, s_gr, s_th, rob_radius and rob_theta
+// are not used).  kOpt compiles the optional behaviours of SURVEY 8(f) N4 in (humans.policy = social_force,
+// random_policy_changing, random_unobservability); the default kernel has none of them.
+template <int G, bool kOpt, int kAgent = AGENT_HUMAN>
 __device__ __forceinline__ float2 orca_group(const CnConfig &cfg, const GroupOps<G> &g, int i, int H,
                                              const float4 *s_pv, const float4 *s_gr, const float *s_th, float2 pref,
                                              float4 rob_pv, float rob_radius, float rob_theta, float4 *s_scratch,
                                              const EnvParams &P, int e)
 {
-    const float4 me = s_pv[i];
-    const float4 me_g = s_gr[i];
+    constexpr bool kRobot = kAgent != AGENT_HUMAN;
+    const float4 me = kRobot ? rob_pv : s_pv[i];
+    const float4 me_g = kRobot ? P.a.rob_gr[e] : s_gr[i];
     const float radius = (float)((double)me_g.z + 0.01 + (double)cfg.orca_safety_space);
     const float max_speed = me_g.w;
     const float prefx = pref.x, prefy = pref.y;
 
-    const int M = H - 1 + (cfg.robot_visible ? 1 : 0);
+    const int M = kRobot ? H : H - 1 + (cfg.robot_visible ? 1 : 0);
     const bool have = g.gl < M;
     float ox = 0.f, oy = 0.f, ovx = 0.f, ovy = 0.f, orad = 0.f;
     double raw_r = 0.0;
     int4 ctr = make_int4(0, 0, 0, 0);
     if (kOpt) ctr = P.a.ctr[e];
-    if (have) {
+    if (kRobot && have) {
+        const size_t hi = (size_t)e * H + g.gl;
+        const float4 b = P.a.hum_bel[hi];
+        ox = b.x; oy = b.y; ovx = b.z; ovy = b.w; raw_r = (double)P.a.hum_br[hi];
+        orad = (float)(raw_r + 0.01 + (double)cfg.orca_safety_space);
+    }
+    if (!kRobot && have) {
         const bool limited = cfg.human_fov < 2.0 * CN_PI;
         const double my_th = (limited && cfg.kinematics != CN_HOLONOMIC) ? (double)s_th[i] : 0.0;
         bool vis = true;
@@ -210,7 +224,7 @@ __device__ __forceinline__ float2 orca_group(const CnConfig &cfg, const GroupOps
         if (!vis) { ox = 7.0f; oy = 7.0f; ovx = 0.0f; ovy = 0.0f; }   // dummy_human, crowd_sim.py:161-163
         orad = (float)(raw_r + 0.01 + (double)cfg.orca_safety_space);
     }
-    if (kOpt && human_policy_of(cfg, ctr.z, e, i) == CN_POLICY_SOCIAL_FORCE) {
+    if (kAgent == AGENT_ROBOT_SF || (kOpt && human_policy_of(cfg, ctr.z, e, i) == CN_POLICY_SOCIAL_FORCE)) {
         // SOCIAL_FORCE.predict (crowd_nav/policy/social_force.py:11-63), Python floats -> fp64.  Lane k owns the push of
         // neighbour slot k; the sum runs in slot order like the reference's loop.
         double tx = 0.0, ty = 0.0;
@@ -1293,6 +1307,58 @@ extern "C" int cn_launch_crowd_step(const EnvParams *P, const CnStepOut *out, co
     case 8: crowd_step_kernel<8, false, 0><<<grid, STEP_THREADS, smem, stream>>>(*P, *out, action, E, auto_reset); break;
     case 16: crowd_step_kernel<16, false, 0><<<grid, STEP_THREADS, smem, stream>>>(*P, *out, action, E, auto_reset); break;
     default: crowd_step_kernel<32, false, 0><<<grid, STEP_THREADS, smem, stream>>>(*P, *out, action, E, auto_reset); break;
+    }
+    return (int)cudaGetLastError();
+}
+
+// ---------------------------------------------------------------------------------------------- K8: model-based robot
+// The action of an ORCA or social-force robot (config robot.policy = orca / social_force): orca.py:64-139 or
+// social_force.py:11-63 with the robot as agent 0 and the H rows of last_human_states (hum_bel / hum_br: what the DS-RNN
+// observation is built from) as the others, in human index order.  One G-lane group per env, lane k owns belief row k;
+// the solve is the humans' own (orca_group), so the arithmetic is the same fp32 / fp64.
+// Reads only the running episode's arrays (never the spares the forked refill writes); writes float32 [N, 2].
+template <int G, int kAgent>
+__global__ void __launch_bounds__(STEP_THREADS)
+robot_act_kernel(const __grid_constant__ EnvParams P, float2 *__restrict__ action)
+{
+    __shared__ __align__(16) float4 s_scr[2 * STEP_THREADS];     // per group: G ranked lines + G projected lines
+    const CnConfig &cfg = P.cfg;
+    const int H = cfg.human_num;
+    GroupOps<G> g;
+    const int lane = threadIdx.x & 31;
+    g.gl = lane % G;
+    g.gbase = lane - g.gl;
+    g.gmask = (G == 32) ? 0xffffffffu : (GroupOps<G>::kLow << g.gbase);
+    const int group = threadIdx.x / G;
+    const int e = blockIdx.x * (STEP_THREADS / G) + group;
+    if (e >= P.n_envs) return;                                  // whole groups only: no lane of a live group leaves
+    const float4 me = P.a.rob_pv[e];
+    const float2 pref = kAgent == AGENT_ROBOT_ORCA ? preferred_velocity(me, P.a.rob_gr[e]) : make_float2(0.f, 0.f);
+    const float2 v = orca_group<G, false, kAgent>(cfg, g, 0, H, nullptr, nullptr, nullptr, pref, me, 0.f, 0.f, s_scr + group * G, P, e);
+    if (g.gl == 0) action[e] = v;
+}
+
+// host launcher (called from c_abi.cu): one launch, no allocation, no synchronisation
+extern "C" int cn_launch_robot_act(const EnvParams *P, int policy, float *action, cudaStream_t stream)
+{
+    const int H = P->cfg.human_num;
+    const int G = pick_group(H);
+    const int grid = (P->n_envs + STEP_THREADS / G - 1) / (STEP_THREADS / G);
+    float2 *out = reinterpret_cast<float2 *>(action);
+    if (policy == CN_POLICY_SOCIAL_FORCE) {
+        switch (G) {
+        case 4: robot_act_kernel<4, AGENT_ROBOT_SF><<<grid, STEP_THREADS, 0, stream>>>(*P, out); break;
+        case 8: robot_act_kernel<8, AGENT_ROBOT_SF><<<grid, STEP_THREADS, 0, stream>>>(*P, out); break;
+        case 16: robot_act_kernel<16, AGENT_ROBOT_SF><<<grid, STEP_THREADS, 0, stream>>>(*P, out); break;
+        default: robot_act_kernel<32, AGENT_ROBOT_SF><<<grid, STEP_THREADS, 0, stream>>>(*P, out); break;
+        }
+    } else {
+        switch (G) {
+        case 4: robot_act_kernel<4, AGENT_ROBOT_ORCA><<<grid, STEP_THREADS, 0, stream>>>(*P, out); break;
+        case 8: robot_act_kernel<8, AGENT_ROBOT_ORCA><<<grid, STEP_THREADS, 0, stream>>>(*P, out); break;
+        case 16: robot_act_kernel<16, AGENT_ROBOT_ORCA><<<grid, STEP_THREADS, 0, stream>>>(*P, out); break;
+        default: robot_act_kernel<32, AGENT_ROBOT_ORCA><<<grid, STEP_THREADS, 0, stream>>>(*P, out); break;
+        }
     }
     return (int)cudaGetLastError();
 }

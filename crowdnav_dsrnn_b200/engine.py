@@ -160,6 +160,24 @@ class CrowdEngine:
         self.launches += self.lib.cn_env_last_launches(self.handle)
         return b
 
+    def robot_act(self, policy, out=None):
+        """Action of a model-based robot on every env from the running state: ORCA.predict / SOCIAL_FORCE.predict with the
+        robot as self and the belief rows last_human_states as the others (cn_env_robot_act) -> device float32 [N, 2],
+        the velocities to pass to step().  `policy`: "orca" / "social_force" (or abi.POLICY_*), on a holonomic engine
+        whatever config.robot.policy is.  `out` (contiguous float32 [N, 2] on this device) gives the result a static
+        address (CUDA graphs)."""
+        code = abi.ROBOT_POLICIES.get(policy, policy) if isinstance(policy, str) else int(policy)
+        if code not in abi.ROBOT_POLICIES.values():
+            raise ValueError("policy must be one of %s, got %r" % (sorted(abi.ROBOT_POLICIES), policy))
+        dev = torch.device("cuda", self.device_index)
+        if out is None:
+            out = torch.empty(self.n, 2, dtype=torch.float32, device=dev)
+        elif out.dtype != torch.float32 or out.device != dev or tuple(out.shape) != (self.n, 2) or not out.is_contiguous():
+            raise ValueError("out must be a contiguous float32 tensor [%d, 2] on %s" % (self.n, dev))
+        _lib.check(self.lib.cn_env_robot_act(self.handle, code, _ptr(out), self._stream()), "cn_env_robot_act")
+        self.launches += self.lib.cn_env_last_launches(self.handle)
+        return out
+
     def join(self):
         """Make the current stream wait for the spare-episode refill forked by the last reset()/step() (the library joins it
         by itself at the next call; an explicit join is needed at the end of a CUDA-graph capture)."""

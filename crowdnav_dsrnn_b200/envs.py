@@ -8,6 +8,7 @@ Returned object (`CrowdVecEnv`):
   .observation_space.spaces / .action_space / .num_envs
   .reset()            -> dict[str, float32 Tensor on device]
   .step(action[N,2])  -> (obs dict, reward CPU float32 Tensor [N,1], done numpy bool [N], infos)
+                         (robot.policy 'orca' / 'social_force': the robot acts by itself and `action` is ignored)
   .step_async / .step_wait / .render(mode="rgb_array") / .get_images / .close
   .venv.envs[0].env   -> object with .global_time .time_step .time_limit .robot.{time_step,v_pref} (evaluation.py:71)
 `infos` is a lazy sequence: `infos[i]` builds the reference-shaped dict
@@ -114,11 +115,15 @@ class _EnvView(object):
 
 class CrowdVecEnv(object):
     def __init__(self, config, num_envs, device, seed=0, phase=None, test_case=-1, env_id_offset=0, nenv=None):
+        # robot.policy 'orca' / 'social_force': every step first asks the model-based robot for its action
+        # (CrowdEngine.robot_act) and the caller's actions are ignored; refused before any CUDA work
+        self.robot_policy = abi.robot_policy_of(config)
         self.config = config
         self.num_envs = int(num_envs)
         self.device = torch.device(device)
         self.engine = CrowdEngine(config, self.num_envs, self.device, phase=phase, seed=seed,
                                   env_id_offset=env_id_offset, nenv=nenv)
+        self._robot_action = None
         self.observation_space, self.action_space = crowd_spaces(config.sim.human_num)
         self._side = bool(config.test.side_preference)
         self._t0 = time.time()
@@ -139,8 +144,15 @@ class CrowdVecEnv(object):
     def step_async(self, actions):
         self._pending = actions
 
+    def _step_engine(self, actions):
+        if self.robot_policy is not None:
+            if self._robot_action is None:
+                self._robot_action = torch.empty(self.num_envs, 2, dtype=torch.float32, device=self.device)
+            actions = self.engine.robot_act(self.robot_policy, out=self._robot_action)
+        return self.engine.step(actions, auto_reset=True)
+
     def step_wait(self):
-        buf = self.engine.step(self._pending, auto_reset=True)
+        buf = self._step_engine(self._pending)
         self._pending = None
         # VecPyTorch.step_wait keeps reward on the CPU and done as a numpy array (envs.py:231-239): both cross PCIe in
         # ONE synchronisation through pinned staging buffers (fresh host tensors are returned, like the reference)
@@ -166,7 +178,7 @@ class CrowdVecEnv(object):
 
     def step_device(self, actions):
         """Tensor-native fast path: everything stays on the GPU, nothing is synchronised."""
-        buf = self.engine.step(actions, auto_reset=True)
+        buf = self._step_engine(actions)
         return buf.obs(), buf.reward, buf.done, buf
 
     def get_images(self, env_ids=None, size=256):
@@ -193,6 +205,4 @@ def make_vec_envs(env_name, seed, num_processes, gamma, log_dir, device, allow_e
         raise NotImplementedError("only CrowdSimDict-v0 is on the hot path (got %r)" % (env_name,))
     if config is None:
         raise ValueError("config is required")
-    if config.robot.policy != "srnn":
-        raise NotImplementedError("robot.policy=%r (only 'srnn' uses the dict observation)" % (config.robot.policy,))
     return CrowdVecEnv(config, num_processes, device, seed=seed, test_case=test_case)

@@ -9,6 +9,9 @@ shows up in the first jerk sample (SM4) of every episode; to reproduce that, eve
 unscored episodes (env k starts at counter k - warmup) and the NEXT one is scored.  The rollout stops when every env
 has finished its scored episode.  Per-step social metrics (SM1-SM6, evaluation.py:155-190) are accumulated on the
 device from the step-info columns.
+
+With a model-based robot (robot.policy = 'orca' / 'social_force') the robot acts by itself inside the vectorised env's
+step: `actor_critic` is None and no forward runs, everything else is the same.
 """
 import math
 
@@ -22,6 +25,11 @@ from .envs import CrowdVecEnv
 @torch.no_grad()
 def evaluate_batched(actor_critic, config, device, episodes=None, seed=None, deterministic=True, warmup_episodes=1,
                      return_episodes=False):
+    robot_policy = abi.robot_policy_of(config)
+    if robot_policy is not None and actor_critic is not None:
+        raise ValueError("robot.policy=%r acts by itself: evaluate it with actor_critic=None" % (config.robot.policy,))
+    if robot_policy is None and actor_critic is None:
+        raise ValueError("robot.policy='srnn' needs the actor_critic that drives it")
     n = int(config.env.test_size if episodes is None else episodes)
     device = torch.device(device)
     venv = CrowdVecEnv(config, n, device, seed=config.env.seed if seed is None else seed, phase="test", nenv=1)
@@ -35,8 +43,9 @@ def evaluate_batched(actor_critic, config, device, episodes=None, seed=None, det
     st["counters"][:, 2] = (ks % size).to(torch.int32)
     eng.set_state(counters=st["counters"])
     obs = eng.reset().obs()
-    hx = {"human_node_rnn": torch.zeros(n, 1, 128, device=device),
-          "human_human_edge_rnn": torch.zeros(n, H + 1, 256, device=device)}
+    hx = None if actor_critic is None else {"human_node_rnn": torch.zeros(n, 1, 128, device=device),
+                                            "human_human_edge_rnn": torch.zeros(n, H + 1, 256, device=device)}
+    action = None
     masks = torch.zeros(n, 1, device=device)
     finished = torch.zeros(n, dtype=torch.bool, device=device)
     ep_idx = torch.zeros(n, dtype=torch.int32, device=device)      # episodes completed so far by each env
@@ -55,7 +64,8 @@ def evaluate_batched(actor_critic, config, device, episodes=None, seed=None, det
     last_pos = obs["robot_node"][:, 0, 0:2].clone()
     last_angle = torch.atan2(obs["temporal_edges"][:, 0, 1], obs["temporal_edges"][:, 0, 0])
     for _ in range((W + 1) * (int(eng.cfg.timeout_step) + 2)):
-        _, action, _, hx = actor_critic.act(obs, hx, masks, deterministic=deterministic)
+        if actor_critic is not None:
+            _, action, _, hx = actor_critic.act(obs, hx, masks, deterministic=deterministic)
         obs, _, done, buf = venv.step_device(action)
         live = ep_idx == W                                          # currently playing the scored episode
         for k in acc:
@@ -138,7 +148,8 @@ def evaluate(actor_critic, ob_rms, eval_envs, num_processes, device, config, log
     triple -- but the `env.test_size` episodes are played as ONE batch on the GPU (`evaluate_batched`), not one after the
     other in `eval_envs` (which is only closed, as the reference does at the end).  Episode k of the reference is env k of
     the batch.  The returned dicts hold one `[episode total]` list per episode (the per-step traces that
-    test.py --study_scenario plots are not kept on the host); `dist_to_goal` is left empty."""
+    test.py --study_scenario plots are not kept on the host); `dist_to_goal` is left empty.  A model-based robot
+    (robot.policy = 'orca' / 'social_force') is evaluated with actor_critic=None."""
     if visualize:
         raise NotImplementedError("rendering is out of scope (SURVEY section 2 row 2)")
     if recurrent_type != "GRU":

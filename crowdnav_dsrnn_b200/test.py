@@ -3,6 +3,10 @@ command-line flags, same model-directory layout (`<model_dir>/configs/train_conf
 same log file name (`<model_dir>/test/model_<ckpt>_test_<name>_.log`, test.py:103-128) and the log lines of
 pytorchBaselines/evaluation.py:283-330; the `env.test_size` test episodes are played as one batch on the GPU.
 
+--robot_policy orca / social_force evaluates a model-based robot instead of a checkpoint: config.robot.policy is
+overridden, no checkpoint is loaded, `--model_dir` still supplies the config and the log directory, and the log file is
+named as if the policy were the checkpoint (`model_orca_test_<name>_.log`).
+
 --viz / --study_scenario need the renderer / per-step traces, which are out of scope (SURVEY section 2 row 2)."""
 import argparse
 import importlib
@@ -52,15 +56,21 @@ def main(argv=None):
     ap.add_argument("--default_config", type=bool, default=True)
     ap.add_argument("--num_threads", type=int, default=1)
     ap.add_argument("--study_scenario", action="store_true")
+    ap.add_argument("--robot_policy", type=str, default=None, choices=["orca", "social_force"],
+                    help="evaluate a model-based robot instead of a checkpoint")
     args = ap.parse_args(argv)
     if args.viz or args.study_scenario:
         raise NotImplementedError("--viz / --study_scenario need the renderer (out of scope, SURVEY section 2 row 2)")
     model_dir = args.model_dir.rstrip("/")
     if os.getcwd() not in sys.path:
         sys.path.insert(0, os.getcwd())
-    if args.test_model is None:                  # test.py:61-81: newest checkpoint of the run
+    if args.robot_policy is not None:
+        args.test_model = args.robot_policy
+    elif args.test_model is None:                # test.py:61-81: newest checkpoint of the run
         args.test_model = sorted(os.listdir(os.path.join(model_dir, "checkpoints")), reverse=True)[0]
     config = _load_config(model_dir, args.default_config)
+    if args.robot_policy is not None:
+        config.robot.policy = args.robot_policy
     log_dir = Path.cwd() / model_dir / "test"
     log_dir.mkdir(parents=True, exist_ok=True)
     log_file = str(log_dir / log_file_name(args.test_model, args.test_name))
@@ -82,14 +92,19 @@ def main(argv=None):
     torch.cuda.manual_seed_all(config.env.seed)
     torch.set_num_threads(args.num_threads)
     device = torch.device("cuda:0")
-    load_path = str(Path.cwd() / model_dir / "checkpoints" / args.test_model)
-    logger.info("Using model %s" % load_path)
+    if args.robot_policy is not None:
+        logger.info("Using robot policy %s" % args.robot_policy)
+    else:
+        load_path = str(Path.cwd() / model_dir / "checkpoints" / args.test_model)
+        logger.info("Using model %s" % load_path)
     envs = make_vec_envs(config.env.env_name, config.env.seed, 1, config.reward.gamma, None, device, allow_early_resets=True,
                          config=config, test_case=args.test_case)
-    actor_critic = Policy(envs.observation_space.spaces, envs.action_space, base_kwargs=config, base=config.robot.policy)
-    actor_critic.load_state_dict(torch.load(load_path, map_location=device))
-    actor_critic.base.nenv = 1
-    actor_critic.to(device)
+    actor_critic = None
+    if args.robot_policy is None:
+        actor_critic = Policy(envs.observation_space.spaces, envs.action_space, base_kwargs=config, base=config.robot.policy)
+        actor_critic.load_state_dict(torch.load(load_path, map_location=device))
+        actor_critic.base.nenv = 1
+        actor_critic.to(device)
     evaluate(actor_critic=actor_critic, ob_rms=False, eval_envs=envs, num_processes=1, device=device, config=config,
              logging=logger, visualize=False, recurrent_type="GRU")
     for h in list(logger.handlers):

@@ -198,6 +198,13 @@ int cn_env_get_state(CnEnv *env, const CnStateView *view, void *stream);
 /* regenerate the observation from the current state without stepping (generate_ob(reset=True) semantics) */
 int cn_env_observe(CnEnv *env, const CnObsOut *obs, void *stream);
 
+/* Action of a model-based robot (robot.policy = orca / social_force): ORCA.predict (orca.py:64-139) or
+ * SOCIAL_FORCE.predict (social_force.py:11-63) with the robot's pre-step state as self and the H belief rows
+ * last_human_states (what the DS-RNN observation is built from) as the others, in human index order -> action_dev
+ * [N,2] float32 velocities, 8-byte aligned, to pass to cn_env_step.  policy: CN_POLICY_ORCA / CN_POLICY_SOCIAL_FORCE;
+ * holonomic envs only (CN_ERR_ARG for a unicycle env).  No allocation, no synchronisation (graph-capturable). */
+int cn_env_robot_act(CnEnv *env, int32_t policy, float *action_dev, void *stream);
+
 /*
  * Frames (render(mode="rgb_array"), crowd_sim.py:1207-1461 without matplotlib): the square [-L/2, L/2]^2 of
  * L = sim.square_width, row 0 at the top (+y up), pixel (i, j) sampled at its centre.  Layers, later over earlier:

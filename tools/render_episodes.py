@@ -1,4 +1,4 @@
-"""Record test episodes of a checkpoint as PNG frames drawn on the GPU (CrowdEngine.render, kernel K7).
+"""Record test episodes of a checkpoint (or of a model-based robot) as PNG frames drawn on the GPU (CrowdEngine.render, K7).
 
 Plays `--episodes k` test episodes in one batch, deterministically, the way `evaluate_batched` starts them (env k plays
 test case k), and renders every step of every env until that env's first episode ends, the last frame showing the end
@@ -6,6 +6,7 @@ test case k), and renders every step of every env until that env's first episode
 with all envs in baselines' tile_images layout.  PNGs are written with stdlib zlib; nothing else is needed.
 
     python tools/render_episodes.py --checkpoint tests/golden/weights_holonomic_27776.npz --episodes 16 --out frames
+    python tools/render_episodes.py --robot_policy orca --episodes 16 --out frames_orca      # no checkpoint: robot.policy
 """
 import argparse
 import os
@@ -32,14 +33,17 @@ def load_weights(path):
 
 @torch.no_grad()
 def record(config, state_dict, episodes, out, size=256, tile=False, device="cuda:0", seed=None, max_steps=None):
-    """Returns {env: number of frames written}."""
+    """Returns {env: number of frames written}.  `state_dict` is None for a model-based robot (config.robot.policy
+    'orca' / 'social_force'), whose action comes from CrowdEngine.robot_act."""
     dev = torch.device(device)
     n = int(episodes)
     venv = CrowdVecEnv(config, n, dev, seed=config.env.seed if seed is None else seed, phase="test", nenv=1)
     eng = venv.engine
-    policy = Policy(venv.observation_space.spaces, venv.action_space, base="srnn", base_kwargs=config)
-    policy.load_state_dict(state_dict)
-    policy = policy.to(dev)
+    policy = None
+    if venv.robot_policy is None:
+        policy = Policy(venv.observation_space.spaces, venv.action_space, base="srnn", base_kwargs=config)
+        policy.load_state_dict(state_dict)
+        policy = policy.to(dev)
     st = eng.get_state()                    # env k plays test case k (evaluate_batched with no warm-up episode)
     ks = torch.arange(n, dtype=torch.int64, device=dev)
     st["counters"][:, 1] = (ks % 4).to(torch.int32)
@@ -67,7 +71,10 @@ def record(config, state_dict, episodes, out, size=256, tile=False, device="cuda
     step = 0
     write(step, np.arange(n))                             # the reset
     while live.any() and step < limit:
-        _, action, _, hx = policy.act(obs, hx, masks, deterministic=True)
+        if policy is None:
+            action = eng.robot_act(venv.robot_policy)
+        else:
+            _, action, _, hx = policy.act(obs, hx, masks, deterministic=True)
         buf = eng.step(action, auto_reset=False)           # a finished env keeps its last state: its final frame shows it
         obs, masks = buf.obs(), buf.not_done
         step += 1
@@ -89,12 +96,16 @@ def main(argv=None):
     ap.add_argument("--humans", type=int, default=None)
     ap.add_argument("--fov", type=float, default=None, help="robot.FOV (multiples of pi)")
     ap.add_argument("--seed", type=int, default=None)
+    ap.add_argument("--robot_policy", default=None, choices=["orca", "social_force"],
+                    help="record a model-based robot instead of the checkpoint")
     args = ap.parse_args(argv)
     check_size(args.size)
     cfg = Config(kinematics=args.kinematics, human_num=args.humans)
     if args.fov is not None:
         cfg.robot.FOV = args.fov
-    written = record(cfg, load_weights(args.checkpoint), args.episodes, args.out, size=args.size, tile=args.tile,
+    if args.robot_policy is not None:
+        cfg.robot.policy = args.robot_policy
+    written = record(cfg, None if args.robot_policy else load_weights(args.checkpoint), args.episodes, args.out, size=args.size, tile=args.tile,
                      seed=args.seed)
     print("wrote %d frames of %d episodes to %s (frames per episode: %s)" % (
         sum(written.values()), len(written), args.out, " ".join(str(written[k]) for k in sorted(written))))
