@@ -1238,6 +1238,13 @@ extern "C" int cn_crowd_step_launches(const EnvParams *P)
     return 1;
 }
 
+// the instantiation of the group form the launcher runs first (the split form's ORCA launch has the same shared memory)
+template <int G>
+static const void *step_kernel_of(bool opt)
+{
+    return opt ? (const void *)crowd_step_kernel<G, true, 0> : (const void *)crowd_step_kernel<G, false, 0>;
+}
+
 // host launcher (called from c_abi.cu)
 extern "C" int cn_launch_crowd_step(const EnvParams *P, const CnStepOut *out, const float *action, int auto_reset, cudaStream_t stream)
 {
@@ -1278,7 +1285,19 @@ extern "C" int cn_launch_crowd_step(const EnvParams *P, const CnStepOut *out, co
     // small batches (BASELINE configs[0], [1]): a CTA is a latency chain of ~E*H/groups solves plus one tail per warp, and
     // there are not enough CTAs to fill the GPU anyway -- spread the envs over at least ~4 CTAs per SM
     if (num_sms > 0 && P->n_envs < E * 4 * num_sms) { E = P->n_envs / (4 * num_sms); E = E < 1 ? 1 : E; }
-    if (const char *dbg = getenv("CN_STEP_ENVS_PER_CTA")) { const int v = atoi(dbg); if (v >= 1 && v <= 64) E = v; }   // tuning knob
+    if (const char *dbg = getenv("CN_STEP_ENVS_PER_CTA")) {          // tuning knob
+        const int v = atoi(dbg);
+        if (v >= 1 && v <= 64) E = v;
+        // the kernel runs with the default 48 KB shared-memory limit (no cudaFuncSetAttribute: more would change the
+        // occupancy of the default shapes), so a value whose E*H humans do not fit beside the kernel's static shared
+        // memory is clamped to the largest that does (E = 43 at H = 20, 27 at H = 32; the default E always fits)
+        const void *k = G == 4 ? step_kernel_of<4>(opt) : G == 8 ? step_kernel_of<8>(opt) : G == 16 ? step_kernel_of<16>(opt) : step_kernel_of<32>(opt);
+        cudaFuncAttributes fa;
+        const cudaError_t rc = cudaFuncGetAttributes(&fa, k);
+        if (rc != cudaSuccess) return (int)rc;
+        const int e_fit = (int)((48 * 1024 - fa.sharedSizeBytes - 2 * STEP_THREADS * 16) / (H * (16 + 16 + 8 + 4)));
+        if (E > e_fit) E = e_fit;
+    }
     const size_t smem = (size_t)E * H * (16 + 16 + 8 + 4) + 2 * STEP_THREADS * 16;
     const int grid = (P->n_envs + E - 1) / E;
     if (opt) {
